@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — Mrays/s of the B200-native voxel raytracer on BASELINE.json's workload.
 
-    python bench.py --gpus N --steps K --warmup W [--impl reference] [--workload c2|c0|c1|c3|c4]
+    python bench.py --gpus N --steps K --warmup W [--impl reference] [--workload c2|c0|c1|c3|c4] [--dump-outputs DIR]
 
 Default workload (the one BASELINE.json's metric is quoted on): a "step" is one full frame (1920x1080 primary
 rays) of the 256^3 mixed-transparent Space (BASELINE.json configs[2], SURVEY.md §8(d) C2) traced through the C ABI
@@ -16,6 +16,9 @@ Prints ONE JSON line (rank 0).  `value` = rays / device time with inputs residen
 region); `roofline` = algorithmic bytes / kernel time vs the measured HBM peak;
 `cpu_baseline` = the oracle (CPU restatement of the reference, all host threads) on a bounded
 sample of the same frame.  `--impl reference` times only that CPU path.
+
+`--dump-outputs DIR` writes what the last timed step computed, as the caller of the GPU path receives it, to
+DIR/<name>.npy (see dump_outputs), so that two builds can be compared output for output on identical inputs.
 """
 import argparse
 import ctypes as C
@@ -49,7 +52,43 @@ def parse_args():
                    help="N>1: 'p2p' = the encode kernel stores its strips straight into rank 0's frame over NVLink "
                         "(CUDA IPC mapped peer memory) and an arrival counter in that memory replaces the collective; "
                         "'p2p-barrier' = the same stores + an NCCL barrier; 'nccl' = packed strips + NCCL gather + reassembly")
-    return p.parse_args()
+    p.add_argument("--dump-outputs", metavar="DIR",
+                   help="after the timed steps, write the outputs of the last one as DIR/<name>.npy (float32/float64)")
+    args = p.parse_args()
+    if args.steps < 1:
+        p.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        # the CPU arm renders a row sample sized by its own timing, so its output is not the same from run to run
+        p.error("--dump-outputs applies to the GPU path, not to --impl reference")
+    return args
+
+
+DUMP_BYTES = 63_000_000   # array data; with the .npy headers the files stay under 64 MB
+
+
+def dump_outputs(out_dir, arrays):
+    """Writes each array as out_dir/<name>.npy: float64 for 64-bit inputs, float32 otherwise (exact for the uint8
+    pixels and light texels).  If they would come to more than DUMP_BYTES, each multi-dimensional array is cut to the
+    same fraction of its records (entries along the last axis, e.g. the RGBA of a pixel), chosen with a fixed seed so that
+    every run keeps the same records: <name>.npy then has shape [k, channels] and <name>_index.npy (float64) holds the
+    flat record indices."""
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {k: np.asarray(v) for k, v in arrays.items()}
+    arrays = {k: a.astype(np.float64 if a.dtype.itemsize == 8 else np.float32) for k, a in arrays.items()}
+    whole = sum(a.nbytes for a in arrays.values())
+    fraction = 1.0
+    if whole > DUMP_BYTES:
+        fixed = sum(a.nbytes for a in arrays.values() if a.ndim < 2)
+        per_record = sum(a.nbytes + 8 * (a.size // a.shape[-1]) for a in arrays.values() if a.ndim >= 2)
+        fraction = (DUMP_BYTES - fixed) / per_record
+    for name, a in arrays.items():
+        if fraction < 1.0 and a.ndim >= 2:
+            records = a.reshape(-1, a.shape[-1])
+            k = int(records.shape[0] * fraction)
+            index = np.sort(np.random.default_rng(0).choice(records.shape[0], k, replace=False))
+            np.save(os.path.join(out_dir, f"{name}_index.npy"), index.astype(np.float64))
+            a = records[index]
+        np.save(os.path.join(out_dir, f"{name}.npy"), a)
 
 
 def make_workload(name):
@@ -271,7 +310,7 @@ def run_light(args):
         u, md = rt.light_edit_and_propagate(cubes, ids, 1)   # H2D: the edit list; blocks until the propagation is done
         st = rt.light_stats()
         img = r.draw() if render else None                   # D2H: the frame
-        return u, st, time.perf_counter() - t0, img
+        return u, md, st, time.perf_counter() - t0, img
 
     for k in range(max(3, args.warmup)):
         step(k, True)
@@ -281,7 +320,7 @@ def run_light(args):
     render_ms = []
     launches = 0
     for k in range(args.steps):
-        u, st, wall, img = step(max(3, args.warmup) + k, True)
+        u, md, st, wall, img = step(max(3, args.warmup) + k, True)
         tot_u += u
         tot_v += st["chart_node_visits"]
         dev_s += st["device_seconds"]
@@ -289,6 +328,9 @@ def run_light(args):
         render_ms.append(img.info.kernel_ms)
         launches += 2 + 7 * st["rounds"] + 4   # edits + tile rebuild; 7 kernels per relaxation round; the 4 kernels of the re-render
     clocks = sampler.stop()
+    if args.dump_outputs:   # the last step's (updates, max difference), the light it left in the Space, its re-render
+        dump_outputs(args.dump_outputs, {"light_update": np.array([u, md], dtype=np.int64),
+                                         "light": rt.light_download(), "frame": img.data})
     value = tot_u / dev_s
     peaks = {}
     try:
@@ -532,6 +574,15 @@ def run_ours(args):
     sampler.mark()
     check(lib.aicb_ctx_stage_timing(ctx.handle, 0))   # the timed frames carry no per-kernel event records
     total_ms = timed(device_step, args.steps)
+    if args.dump_outputs and rank == 0:   # the frame the last timed step delivered to rank 0
+        if world == 1:
+            last = d_out[:n_local].cpu()
+        elif gather_mode == "p2p":
+            last = torch.empty((h * w, 4), dtype=torch.uint8).pin_memory()
+            peer.read(last, stream.cuda_stream)
+        else:
+            last = frame.cpu()
+        dump_outputs(args.dump_outputs, {"frame": last.numpy().reshape(h, w, 4)})
     # kernel-only duration of the last frame from the library's own events (same stream); a frame that overflowed its
     # hit stream inside the timed region would make this call fail (AICB_ERR_RETRY) and with it the run
     check(lib.aicb_render_finish(rt.handle, C.byref(info)))
