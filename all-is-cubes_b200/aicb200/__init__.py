@@ -116,6 +116,15 @@ def load_library() -> C.CDLL:
     lib.aicb_group_scene_update_cubes.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_size_t]
     lib.aicb_group_render_srgb8.argtypes = [C.c_void_p, C.POINTER(abi.CameraData), C.POINTER(abi.Options), C.c_void_p,
                                             C.c_size_t, C.POINTER(abi.RenderInfo)]
+    lib.aicb_group_scene_update_blocks.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_size_t]
+    lib.aicb_group_scene_upload_light.argtypes = [C.c_void_p, C.c_void_p, C.c_size_t]
+    lib.aicb_group_light_fast_evaluate.argtypes = [C.c_void_p]
+    lib.aicb_group_light_evaluate.argtypes = [C.c_void_p, C.c_uint8, C.POINTER(C.c_uint64), C.POINTER(C.c_uint8),
+                                              C.POINTER(C.c_uint64)]
+    lib.aicb_group_light_edit_and_propagate.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_size_t, C.c_uint8,
+                                                        C.POINTER(C.c_uint64), C.POINTER(C.c_uint8)]
+    lib.aicb_group_light_download.argtypes = [C.c_void_p, C.c_int, C.c_void_p, C.c_size_t]
+    lib.aicb_group_light_stats.argtypes = [C.c_void_p, C.c_int, C.POINTER(C.c_uint64)]
     lib.aicb_light_chart.argtypes = [C.c_void_p, C.c_void_p]
     lib.aicb_light_chart.restype = C.c_uint32
     lib.aicb_light_fast_evaluate.argtypes = [C.c_void_p]
@@ -726,14 +735,18 @@ def print_space(space: "Space", direction, block_chars: dict, rt: "SpaceRaytrace
 
 class DeviceGroup:
     """Several GPUs driven from this one process through the C ABI (csrc/group.cu): scene replicated, frame cut into
-    interleaved row strips, pixels stored straight into device 0's frame over NVLink."""
+    interleaved row strips, pixels stored straight into device 0's frame over NVLink.  Light propagation runs on the
+    whole group, each member relaxing its own slab of the volume (csrc/light.cu); the light methods are
+    SpaceRaytracer's."""
 
     def __init__(self, device_ids):
         ids = (C.c_int * len(device_ids))(*[int(d) for d in device_ids])
         h = C.c_void_p()
         _check(load_library().aicb_group_create(ids, len(device_ids), C.byref(h)))
         self.handle = h
+        self.size = len(device_ids)
         self.scene = None
+        self.space = None
 
     def update(self, space: "Space"):
         if self.scene:
@@ -744,6 +757,57 @@ class DeviceGroup:
         _check(load_library().aicb_group_scene_create(self.handle, C.byref(desc), C.byref(h)))
         del keep
         self.scene = h
+        self.space = space
+
+    def update_cubes(self, cubes: np.ndarray, block_ids: np.ndarray, light: Optional[np.ndarray] = None):
+        c = np.ascontiguousarray(cubes, dtype=np.int32).reshape(-1, 3)
+        ids = np.ascontiguousarray(block_ids, dtype=np.uint16)
+        lt = None if light is None else np.ascontiguousarray(light, dtype=np.uint8).reshape(-1, 4)
+        _check(load_library().aicb_group_scene_update_cubes(self.scene, c.ctypes.data, ids.ctypes.data,
+                                                            lt.ctypes.data if lt is not None else None, c.shape[0]))
+
+    def update_blocks(self, indices, blocks):
+        idx = np.ascontiguousarray(indices, dtype=np.uint16)
+        arr = (abi.BlockDesc * len(blocks))()
+        for i, b in enumerate(blocks):
+            fill_block_desc(arr[i], b)
+        _check(load_library().aicb_group_scene_update_blocks(self.scene, idx.ctypes.data, arr, len(blocks)))
+
+    def upload_light(self, light: np.ndarray):
+        lt = np.ascontiguousarray(light, dtype=np.uint8).reshape(-1, 4)
+        _check(load_library().aicb_group_scene_upload_light(self.scene, lt.ctypes.data, lt.shape[0]))
+
+    def light_fast_evaluate(self):
+        _check(load_library().aicb_group_light_fast_evaluate(self.scene))
+
+    def light_evaluate(self, epsilon: int = 0):
+        """-> (updates, max_difference, chart_node_visits), summed over the members"""
+        n, md, nv = C.c_uint64(0), C.c_uint8(0), C.c_uint64(0)
+        _check(load_library().aicb_group_light_evaluate(self.scene, epsilon, C.byref(n), C.byref(md), C.byref(nv)))
+        return int(n.value), int(md.value), int(nv.value)
+
+    def light_edit_and_propagate(self, cubes: np.ndarray, block_ids: np.ndarray, epsilon: int = 0):
+        """-> (updates, max_difference)"""
+        c = np.ascontiguousarray(cubes, dtype=np.int32).reshape(-1, 3)
+        ids = np.ascontiguousarray(block_ids, dtype=np.uint16)
+        n, md = C.c_uint64(0), C.c_uint8(0)
+        _check(load_library().aicb_group_light_edit_and_propagate(self.scene, c.ctypes.data, ids.ctypes.data, c.shape[0],
+                                                                  epsilon, C.byref(n), C.byref(md)))
+        return int(n.value), int(md.value)
+
+    def light_download(self, member: int = 0) -> np.ndarray:
+        """The light replica of one member (a position in the group, not a device id)."""
+        out = np.zeros(self.space.size + (4,), dtype=np.uint8)
+        _check(load_library().aicb_group_light_download(self.scene, member, out.ctypes.data, out.size // 4))
+        return out
+
+    def light_stats(self, member: Optional[int] = None) -> dict:
+        """Counters of the last propagation: the group's (updates and visits summed, the slowest member's time) or
+        one member's own."""
+        out = (C.c_uint64 * 4)()
+        _check(load_library().aicb_group_light_stats(self.scene, -1 if member is None else member, out))
+        return {"cube_updates": int(out[0]), "chart_node_visits": int(out[1]), "rounds": int(out[2]),
+                "device_seconds": int(out[3]) * 1e-6}
 
     def draw(self, camera: "Camera", options: "GraphicsOptions") -> "Rendering":
         w, h = camera.data.fb_width, camera.data.fb_height

@@ -162,4 +162,11 @@ EXPORTED_SYMBOLS = [
     "aicb_group_scene_destroy",
     "aicb_group_scene_update_cubes",
     "aicb_group_render_srgb8",
+    "aicb_group_scene_update_blocks",
+    "aicb_group_scene_upload_light",
+    "aicb_group_light_fast_evaluate",
+    "aicb_group_light_evaluate",
+    "aicb_group_light_edit_and_propagate",
+    "aicb_group_light_download",
+    "aicb_group_light_stats",
 ]

@@ -11,20 +11,6 @@
 
 #include "internal.h"
 
-struct aicb_group {
-    std::vector<aicb_ctx *> ctx;
-    std::vector<cudaEvent_t> done;   // per device: its strips of the current frame are in device 0's frame
-    void *d_frame = nullptr;         // on device 0
-    size_t frame_pixels = 0;
-    void *h_stage = nullptr;         // pinned staging for pageable destinations
-    size_t h_stage_bytes = 0;
-};
-
-struct aicb_group_scene {
-    aicb_group *group = nullptr;
-    std::vector<aicb_scene *> scene;
-};
-
 static const uint32_t GROUP_STRIP_ROWS = 16;
 
 extern "C" {
@@ -37,10 +23,9 @@ void aicb_group_destroy(aicb_group *g) {
         if (g->h_stage) cudaFreeHost(g->h_stage);
     }
     for (size_t i = 0; i < g->ctx.size(); i++) {
-        if (g->done[i]) {
-            cudaSetDevice(g->ctx[i]->device);
-            cudaEventDestroy(g->done[i]);
-        }
+        cudaSetDevice(g->ctx[i]->device);
+        if (g->done[i]) cudaEventDestroy(g->done[i]);
+        if (i < g->light_barrier.size() && g->light_barrier[i]) cudaEventDestroy(g->light_barrier[i]);
         aicb_ctx_destroy(g->ctx[i]);
     }
     delete g;
@@ -119,6 +104,26 @@ aicb_status aicb_group_scene_update_cubes(aicb_group_scene *gs, const int32_t (*
     if (!gs) return aicb_fail(AICB_ERR_INVALID, "NULL argument");
     for (aicb_scene *s : gs->scene) {
         aicb_status st = aicb_scene_update_cubes(s, cubes, ids, light, n);
+        if (st != AICB_OK) return st;
+    }
+    return AICB_OK;
+}
+
+// Both validate before they change anything, and every replica holds the same state: a call that fails on member 0
+// fails there, before any replica changed.
+aicb_status aicb_group_scene_update_blocks(aicb_group_scene *gs, const uint16_t *indices, const aicb_block_desc *descs, size_t n) {
+    if (!gs) return aicb_fail(AICB_ERR_INVALID, "NULL argument");
+    for (aicb_scene *s : gs->scene) {
+        aicb_status st = aicb_scene_update_blocks(s, indices, descs, n);
+        if (st != AICB_OK) return st;
+    }
+    return AICB_OK;
+}
+
+aicb_status aicb_group_scene_upload_light(aicb_group_scene *gs, const uint8_t (*light)[4], size_t n_texels) {
+    if (!gs) return aicb_fail(AICB_ERR_INVALID, "NULL argument");
+    for (aicb_scene *s : gs->scene) {
+        aicb_status st = aicb_scene_upload_light(s, light, n_texels);
         if (st != AICB_OK) return st;
     }
     return AICB_OK;

@@ -116,3 +116,23 @@ struct aicb_scene {
     uint32_t light_max_distance = 0;
     uint64_t light_stats[4] = {0, 0, 0, 0};  // last propagation: cube updates, chart node visits, rounds queued, device microseconds
 };
+
+// One process, several GPUs (group.cu renders, light.cu propagates light): one aicb_ctx per member, the scene
+// replicated on each of them.
+struct aicb_group {
+    std::vector<aicb_ctx *> ctx;
+    std::vector<cudaEvent_t> done;   // per device: its strips of the current frame are in device 0's frame
+    void *d_frame = nullptr;         // on device 0
+    size_t frame_pixels = 0;
+    void *h_stage = nullptr;         // pinned staging for pageable destinations
+    size_t h_stage_bytes = 0;
+    // group light propagation (light.cu), set up on its first call
+    bool light_peers_ready = false;          // peer access (with native atomics) between every pair of member devices
+    std::vector<cudaEvent_t> light_barrier;  // per member: its arrival at a round's barrier (member 0's: the release)
+};
+
+struct aicb_group_scene {
+    aicb_group *group = nullptr;
+    std::vector<aicb_scene *> scene;
+    uint64_t light_stats[4] = {0, 0, 0, 0};  // last group propagation: updates and visits summed, rounds, slowest member's time
+};

@@ -702,10 +702,8 @@ bool use_chain_walk() {
     return !(e && std::strcmp(e, "lockstep") == 0);
 }
 
-// evaluate_light (space.rs:1496-1527): rounds until the highest queued priority is <= from_difference(epsilon)
-aicb_status propagate(aicb_scene *s, uint8_t epsilon, uint64_t *updates_done, uint8_t *max_diff, uint64_t *node_visits) {
-    aicb_ctx *ctx = s->ctx;
-    cudaStream_t st = ctx->stream;
+// the parameters of a propagation's rounds
+LightParams propagate_params(aicb_scene *s, uint8_t epsilon) {
     LightParams P = make_params(s);
     P.epsilon_priority = (uint32_t)epsilon / 2 + 1;
     {
@@ -724,6 +722,14 @@ aicb_status propagate(aicb_scene *s, uint8_t epsilon, uint64_t *updates_done, ui
         if (P.batches_per_warp < 1) P.batches_per_warp = 1;
         if (P.min_batch_width < 1) P.min_batch_width = 1;
     }
+    return P;
+}
+
+// evaluate_light (space.rs:1496-1527): rounds until the highest queued priority is <= from_difference(epsilon)
+aicb_status propagate(aicb_scene *s, uint8_t epsilon, uint64_t *updates_done, uint8_t *max_diff, uint64_t *node_visits) {
+    aicb_ctx *ctx = s->ctx;
+    cudaStream_t st = ctx->stream;
+    const LightParams P = propagate_params(s, epsilon);
     const int blocks = ctx->num_sms * 8;
     const int wide = ctx->num_sms * 8;    // 128-thread blocks of the lockstep kernels (one warp per 32 list entries, grid-stride)
     const uint32_t n_tiles = (uint32_t)((s->volume + LIGHT_TILE - 1) / LIGHT_TILE);
@@ -774,6 +780,82 @@ aicb_status propagate(aicb_scene *s, uint8_t epsilon, uint64_t *updates_done, ui
     if (updates_done) *updates_done = total;
     if (max_diff) *max_diff = (uint8_t)maxd;
     if (node_visits) *node_visits = visits;
+    return AICB_OK;
+}
+
+
+// Mutation::set x n (space.rs:1346-1352 -> side_effects_of_set -> modified_cube_needs_update, updater.rs:135-173):
+// validates every edit, then applies them in order to the host mirror and returns what the device has to change.
+// Nothing changes when an edit is invalid.
+aicb_status edit_ops(aicb_scene *s, const int32_t (*cubes)[3], const uint16_t *new_ids, size_t n_edits, std::vector<EditOp> *out) {
+    const DeviceScene &ds = s->ds;
+    auto index_of = [&](int x, int y, int z, uint32_t *idx) {
+        uint32_t dx = (uint32_t)(x - ds.lo[0]), dy = (uint32_t)(y - ds.lo[1]), dz = (uint32_t)(z - ds.lo[2]);
+        if (dx >= (uint32_t)ds.size[0] || dy >= (uint32_t)ds.size[1] || dz >= (uint32_t)ds.size[2]) return false;
+        *idx = (dx * (uint32_t)ds.size[1] + dy) * (uint32_t)ds.size[2] + dz;
+        return true;
+    };
+    std::unordered_map<uint32_t, EditOp> ops;
+    auto op_of = [&](uint32_t idx) -> EditOp & {
+        auto it = ops.find(idx);
+        if (it == ops.end()) {
+            EditOp o;
+            std::memset(&o, 0, sizeof o);
+            o.idx = idx;
+            o.cell = 0xffffffffu;
+            it = ops.emplace(idx, o).first;
+        }
+        return it->second;
+    };
+    // validate everything before the host mirror (or anything else) changes
+    for (size_t i = 0; i < n_edits; i++) {
+        uint32_t idx;
+        if (!index_of(cubes[i][0], cubes[i][1], cubes[i][2], &idx)) return aicb_fail(AICB_ERR_INVALID, "cube out of bounds");
+        if (new_ids[i] >= s->h_block_light.size()) return aicb_fail(AICB_ERR_INVALID, "block id out of range");
+    }
+    for (size_t i = 0; i < n_edits; i++) {
+        uint32_t idx;
+        index_of(cubes[i][0], cubes[i][1], cubes[i][2], &idx);
+        if (s->h_ids[idx] == new_ids[i]) continue;  // Mutation::set of the same block changes nothing
+        s->h_ids[idx] = new_ids[i];
+        EditOp &o = op_of(idx);
+        o.cell = ds.wide_cells ? (new_ids[i] | ((uint32_t)s->block_kind[new_ids[i]] << 16))
+                               : (new_ids[i] | ((uint32_t)s->block_kind[new_ids[i]] << 14));
+        const uint32_t fl = s->h_block_light[new_ids[i]];
+        if ((fl & LB_ALL_OPAQUE) && !(fl & LB_EMISSIVE)) {  // opaque_for_light_computation
+            o.set_opaque = 1;
+            o.pending_op = 1;
+        } else {
+            o.pending_op = 2;
+        }
+        for (int f = 0; f < 6; f++) {
+            const int sgn = (f < 3) ? -1 : 1, a = f % 3;
+            uint32_t nidx;
+            if (!index_of(cubes[i][0] + (a == 0 ? sgn : 0), cubes[i][1] + (a == 1 ? sgn : 0), cubes[i][2] + (a == 2 ? sgn : 0), &nidx))
+                continue;
+            const int opp = (f < 3) ? f + 3 : f - 3;
+            if (!((s->h_block_light[s->h_ids[nidx]] >> opp) & 1u)) op_of(nidx).pending_op = 2;
+        }
+    }
+    out->clear();
+    out->reserve(ops.size());
+    for (auto &kv : ops) out->push_back(kv.second);
+    return AICB_OK;
+}
+
+// the device side of edit_ops: cells, light and queue bytes of the edited cubes and their neighbours
+aicb_status apply_edit_ops(aicb_scene *s, const std::vector<EditOp> &flat) {
+    if (flat.empty()) return AICB_OK;
+    EditOp *d_ops = nullptr;
+    CU(cudaMalloc(&d_ops, flat.size() * sizeof(EditOp)));
+    cudaError_t e = cudaMemcpyAsync(d_ops, flat.data(), flat.size() * sizeof(EditOp), cudaMemcpyHostToDevice, s->ctx->stream);
+    if (e == cudaSuccess) {
+        LightParams P = make_params(s);
+        k_edits<<<(unsigned)((flat.size() + 127) / 128), 128, 0, s->ctx->stream>>>(P, d_ops, (uint32_t)flat.size(), s->ds.wide_cells);
+        e = cudaStreamSynchronize(s->ctx->stream);
+    }
+    cudaFree(d_ops);
+    if (e != cudaSuccess) return aicb_cuda_fail(e, "light edits");
     return AICB_OK;
 }
 
@@ -940,68 +1022,11 @@ aicb_status aicb_light_edit_and_propagate(aicb_scene *s, const int32_t (*cubes)[
     CU(cudaSetDevice(s->ctx->device));
     aicb_status st = ensure_light_state(s);
     if (st != AICB_OK) return st;
-    const DeviceScene &ds = s->ds;
-    auto index_of = [&](int x, int y, int z, uint32_t *idx) {
-        uint32_t dx = (uint32_t)(x - ds.lo[0]), dy = (uint32_t)(y - ds.lo[1]), dz = (uint32_t)(z - ds.lo[2]);
-        if (dx >= (uint32_t)ds.size[0] || dy >= (uint32_t)ds.size[1] || dz >= (uint32_t)ds.size[2]) return false;
-        *idx = (dx * (uint32_t)ds.size[1] + dy) * (uint32_t)ds.size[2] + dz;
-        return true;
-    };
-    std::unordered_map<uint32_t, EditOp> ops;
-    auto op_of = [&](uint32_t idx) -> EditOp & {
-        auto it = ops.find(idx);
-        if (it == ops.end()) {
-            EditOp o;
-            std::memset(&o, 0, sizeof o);
-            o.idx = idx;
-            o.cell = 0xffffffffu;
-            it = ops.emplace(idx, o).first;
-        }
-        return it->second;
-    };
-    // validate everything before the host mirror (or anything else) changes
-    for (size_t i = 0; i < n_edits; i++) {
-        uint32_t idx;
-        if (!index_of(cubes[i][0], cubes[i][1], cubes[i][2], &idx)) return aicb_fail(AICB_ERR_INVALID, "cube out of bounds");
-        if (new_ids[i] >= s->h_block_light.size()) return aicb_fail(AICB_ERR_INVALID, "block id out of range");
-    }
-    for (size_t i = 0; i < n_edits; i++) {
-        uint32_t idx;
-        index_of(cubes[i][0], cubes[i][1], cubes[i][2], &idx);
-        if (s->h_ids[idx] == new_ids[i]) continue;  // Mutation::set of the same block changes nothing
-        s->h_ids[idx] = new_ids[i];
-        EditOp &o = op_of(idx);
-        o.cell = ds.wide_cells ? (new_ids[i] | ((uint32_t)s->block_kind[new_ids[i]] << 16))
-                               : (new_ids[i] | ((uint32_t)s->block_kind[new_ids[i]] << 14));
-        const uint32_t fl = s->h_block_light[new_ids[i]];
-        if ((fl & LB_ALL_OPAQUE) && !(fl & LB_EMISSIVE)) {  // opaque_for_light_computation
-            o.set_opaque = 1;
-            o.pending_op = 1;
-        } else {
-            o.pending_op = 2;
-        }
-        for (int f = 0; f < 6; f++) {
-            const int sgn = (f < 3) ? -1 : 1, a = f % 3;
-            uint32_t nidx;
-            if (!index_of(cubes[i][0] + (a == 0 ? sgn : 0), cubes[i][1] + (a == 1 ? sgn : 0), cubes[i][2] + (a == 2 ? sgn : 0), &nidx))
-                continue;
-            const int opp = (f < 3) ? f + 3 : f - 3;
-            if (!((s->h_block_light[s->h_ids[nidx]] >> opp) & 1u)) op_of(nidx).pending_op = 2;
-        }
-    }
-    if (!ops.empty()) {
-        std::vector<EditOp> flat;
-        flat.reserve(ops.size());
-        for (auto &kv : ops) flat.push_back(kv.second);
-        EditOp *d_ops = nullptr;
-        CU(cudaMalloc(&d_ops, flat.size() * sizeof(EditOp)));
-        CU(cudaMemcpyAsync(d_ops, flat.data(), flat.size() * sizeof(EditOp), cudaMemcpyHostToDevice, s->ctx->stream));
-        LightParams P = make_params(s);
-        k_edits<<<(unsigned)((flat.size() + 127) / 128), 128, 0, s->ctx->stream>>>(P, d_ops, (uint32_t)flat.size(), ds.wide_cells);
-        cudaError_t e = cudaStreamSynchronize(s->ctx->stream);
-        cudaFree(d_ops);
-        if (e != cudaSuccess) return aicb_cuda_fail(e, "light edits");
-    }
+    std::vector<EditOp> ops;
+    st = edit_ops(s, cubes, new_ids, n_edits, &ops);
+    if (st != AICB_OK) return st;
+    st = apply_edit_ops(s, ops);
+    if (st != AICB_OK) return st;
     return propagate(s, epsilon, updates_done, max_diff, nullptr);
 }
 
@@ -1023,3 +1048,433 @@ aicb_status aicb_light_stats(const aicb_scene *s, uint64_t out[4]) {
     return AICB_OK;
 }
 }
+
+// ---------------------------------------------------------------------------------------------
+// light propagation on a device group (aicb_group_light_*): the relaxation sharded by slabs
+// ---------------------------------------------------------------------------------------------
+// Every member holds a full replica of the scene, its light and its queue.  Member i owns the queue tiles
+// [tile_lo[i], tile_lo[i + 1]) (an even split of whole LIGHT_TILE tiles: a slab along x in the Z-major layout, possibly
+// empty); only the owner gathers, computes and applies its cubes.  A round keeps the single-scene round's meaning
+// (propagate()) with barriers (B) between its steps, all stream-ordered through member 0 (no device-side waits):
+//   find_max over the member's queue            B1
+//   clear the queue outside the member's tiles, round priority := the members' maximum, gather, compute (the member's
+//   full replica is read)                       B2  (no replica is written while a peer may still read it)
+//   apply: the owner stores each changed texel into every replica     B3
+//   guess the Uninitialized neighbours (PackedLight::guess): a CAS on the replica of the neighbour's owner   B4
+//   copy guessed texels from their owner into the other replicas; mark (the dependency re-queue) into the member's
+//   full-size queue                             B5
+//   merge: each owner takes the byte-wise maximum of its peers' queue bytes in its own tiles.
+// Between the members' queues: outside its tiles a member's queue only ever holds marks already merged into their
+// owners (so its find_max still yields the global maximum) and is cleared after B1, before that member gathers.
+namespace {
+
+constexpr uint32_t GROUP_LIGHT_MAX = 16;   // members of a propagating group
+
+struct GroupPeers {
+    uint32_t *light[GROUP_LIGHT_MAX];       // every member's replica (device pointers, peer-mapped)
+    uint8_t *pending[GROUP_LIGHT_MAX];
+    uint32_t *tile_max[GROUP_LIGHT_MAX];
+    uint32_t *scalars[GROUP_LIGHT_MAX];
+    uint32_t tile_lo[GROUP_LIGHT_MAX + 1];  // member i owns the tiles [tile_lo[i], tile_lo[i + 1])
+    uint32_t n, self;
+};
+
+__device__ __forceinline__ uint32_t owner_of(const GroupPeers &G, uint32_t idx) {
+    const uint32_t tile = idx / LIGHT_TILE;
+    uint32_t o = G.n - 1;
+    while (o > 0 && tile < G.tile_lo[o]) o--;
+    return o;
+}
+
+// after B1: the queue outside the member's own tiles (already merged into their owners) is cleared
+__global__ void __launch_bounds__(256) k_group_clear_foreign(const LightParams P, const GroupPeers G, uint32_t n_tiles) {
+    const uint32_t lo = G.tile_lo[G.self], hi = G.tile_lo[G.self + 1];
+    const uint32_t n_words = (P.volume + 3) / 4;
+    for (uint32_t tile = blockIdx.x; tile < n_tiles; tile += gridDim.x) {
+        if ((tile >= lo && tile < hi) || P.tile_max[tile] == 0) continue;   // (block-uniform)
+        const uint32_t w = tile * (LIGHT_TILE / 4) + threadIdx.x;
+        if (w < n_words) ((uint32_t *)P.pending)[w] = 0u;
+        __syncthreads();   // every thread has read the tile's bound
+        if (threadIdx.x == 0) P.tile_max[tile] = 0u;
+    }
+}
+
+// after B1: the round's priority is the highest over the members.  A peer may raise its own [1] to the same maximum
+// while it is read here; either value yields the same maximum.
+__global__ void k_group_max(const LightParams P, const GroupPeers G) {
+    if (threadIdx.x >= G.n) return;
+    const uint32_t m = *(volatile const uint32_t *)(G.scalars[threadIdx.x] + 1);
+    if (m) atomicMax(P.scalars + 1, m);
+}
+
+// after B2: apply_light_update (updater.rs:295-363) for the member's own cubes, stored into every replica; the
+// guesses of k_apply are k_group_guess, the dependency re-queue is k_walk_chains<true> / k_mark
+__global__ void k_group_apply(const LightParams P, const GroupPeers G) {
+    const uint32_t n = P.scalars[0];
+    for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) {
+        const uint32_t idx = P.list[i];
+        const uint32_t old = P.scene.light[idx], nv = P.new_light[i];
+        const int d = difference_priority(nv, old);
+        P.diff[i] = (uint8_t)d;
+        atomicAdd(P.scalars + 3, 1u);
+        if (d > 0) {
+            for (uint32_t m = 0; m < G.n; m++) G.light[m][idx] = nv;
+            atomicMax(P.scalars + 2, (uint32_t)d);
+        }
+    }
+}
+
+// after B3: PackedLight::guess for the Uninitialized neighbours of the member's changed cubes, as in k_apply, with
+// the CAS on the neighbour's owner's replica (one winner per texel whichever member guesses)
+__global__ void k_group_guess(const LightParams P, const GroupPeers G) {
+    const uint32_t n = P.scalars[0];
+    const float *lut = P.scene.tables;
+    for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) {
+        if (P.diff[i] == 0) continue;
+        const uint32_t nv = P.new_light[i];
+        int x, y, z;
+        cube_of(P.scene, P.list[i], x, y, z);
+#pragma unroll
+        for (int f = 0; f < 6; f++) {
+            const int s = (f < 3) ? -1 : 1, a = f % 3;
+            uint32_t nidx;
+            if (!cube_index(P.scene, x + (a == 0 ? s : 0), y + (a == 1 ? s : 0), z + (a == 2 ? s : 0), &nidx)) continue;
+            uint32_t *owner = G.light[owner_of(G, nidx)];
+            const uint32_t nl = owner[nidx];
+            if ((nl >> 24) != 0) continue;            // only LightStatus::Uninitialized neighbours
+            if (nl == nv) continue;
+            if (__ldg(&P.blocks[block_id_at(P.scene, nidx)].flags) & LB_ALL_OPAQUE) continue;
+            const uint32_t g = scalar_in_t(lut, lut[nv & 255]) | (scalar_in_t(lut, lut[(nv >> 8) & 255]) << 8) | (scalar_in_t(lut, lut[(nv >> 16) & 255]) << 16);
+            atomicCAS(owner + nidx, nl, g);
+        }
+    }
+}
+
+// after B4: the Uninitialized neighbours of the member's changed cubes (every texel a guess may have changed) are
+// copied from their owner's replica into the others.  Several members may store one texel: all store the same value.
+__global__ void k_group_broadcast(const LightParams P, const GroupPeers G) {
+    const uint32_t n = P.scalars[0];
+    for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) {
+        if (P.diff[i] == 0) continue;
+        int x, y, z;
+        cube_of(P.scene, P.list[i], x, y, z);
+        for (int f = 0; f < 6; f++) {
+            const int s = (f < 3) ? -1 : 1, a = f % 3;
+            uint32_t nidx;
+            if (!cube_index(P.scene, x + (a == 0 ? s : 0), y + (a == 1 ? s : 0), z + (a == 2 ? s : 0), &nidx)) continue;
+            const uint32_t o = owner_of(G, nidx);
+            const uint32_t v = G.light[o][nidx];
+            if ((v >> 24) != 0) continue;
+            for (uint32_t m = 0; m < G.n; m++)
+                if (m != o) G.light[m][nidx] = v;
+        }
+    }
+}
+
+// after B5: the owner takes the byte-wise maximum of its peers' queue bytes in its own tiles (only the tiles a peer's
+// bound says hold something)
+__global__ void __launch_bounds__(256) k_group_merge(const LightParams P, const GroupPeers G) {
+    const uint32_t lo = G.tile_lo[G.self], hi = G.tile_lo[G.self + 1];
+    const uint32_t n_words = (P.volume + 3) / 4;
+    for (uint32_t tile = lo + blockIdx.x; tile < hi; tile += gridDim.x) {
+        const uint32_t w = tile * (LIGHT_TILE / 4) + threadIdx.x;
+        uint32_t v = w < n_words ? ((const uint32_t *)P.pending)[w] : 0u;
+        uint32_t tm = 0;
+        for (uint32_t p = 0; p < G.n; p++) {
+            if (p == G.self) continue;
+            const uint32_t ptm = G.tile_max[p][tile];   // (block-uniform)
+            if (ptm == 0) continue;
+            tm = max(tm, ptm);
+            if (w < n_words) v = __vmaxu4(v, ((const uint32_t *)G.pending[p])[w]);
+        }
+        if (tm) {
+            if (w < n_words) ((uint32_t *)P.pending)[w] = v;
+            if (threadIdx.x == 0 && P.tile_max[tile] < tm) P.tile_max[tile] = tm;
+        }
+    }
+}
+
+// Peer access between every pair of distinct member devices, with native atomics (k_group_guess); members on one
+// device need neither.  Once per group.
+aicb_status group_light_setup(aicb_group *g) {
+    if (g->light_peers_ready) return AICB_OK;
+    const size_t n = g->ctx.size();
+    if (n > GROUP_LIGHT_MAX) return aicb_fail(AICB_ERR_UNSUPPORTED, "light propagation on a group of more than 16 members");
+    for (size_t a = 0; a < n; a++)
+        for (size_t b = 0; b < n; b++) {
+            const int da = g->ctx[a]->device, db = g->ctx[b]->device;
+            if (da == db) continue;
+            int can = 0, atomics = 0;
+            CU(cudaDeviceCanAccessPeer(&can, da, db));
+            CU(cudaDeviceGetP2PAttribute(&atomics, cudaDevP2PAttrNativeAtomicSupported, da, db));
+            if (!can || !atomics)
+                return aicb_fail(AICB_ERR_UNSUPPORTED, "group light propagation needs peer access with native atomics between every pair of devices");
+            CU(cudaSetDevice(da));
+            cudaError_t e = cudaDeviceEnablePeerAccess(db, 0);
+            if (e == cudaErrorPeerAccessAlreadyEnabled) { cudaGetLastError(); e = cudaSuccess; }
+            if (e != cudaSuccess) return aicb_cuda_fail(e, "cudaDeviceEnablePeerAccess");
+        }
+    if (g->light_barrier.size() != n) {
+        g->light_barrier.assign(n, nullptr);
+        for (size_t i = 0; i < n; i++) {
+            CU(cudaSetDevice(g->ctx[i]->device));
+            CU(cudaEventCreateWithFlags(&g->light_barrier[i], cudaEventDisableTiming));
+        }
+    }
+    g->light_peers_ready = true;
+    return AICB_OK;
+}
+
+// evaluate_light on a group of two or more members (the caller holds every member's lock and has set up the light
+// state of every replica)
+aicb_status group_propagate(aicb_group_scene *gs, uint8_t epsilon, uint64_t *updates_done, uint8_t *max_diff, uint64_t *node_visits) {
+    aicb_group *g = gs->group;
+    const uint32_t n = (uint32_t)gs->scene.size();
+    aicb_status st = group_light_setup(g);
+    if (st != AICB_OK) return st;
+    aicb_scene *s0 = gs->scene[0];
+    const uint32_t n_tiles = (uint32_t)((s0->volume + LIGHT_TILE - 1) / LIGHT_TILE);
+    GroupPeers base;
+    std::memset(&base, 0, sizeof base);
+    base.n = n;
+    for (uint32_t i = 0; i < n; i++) {
+        aicb_scene *s = gs->scene[i];
+        base.light[i] = s->d_light;
+        base.pending[i] = s->d_pending;
+        base.tile_max[i] = s->d_tile_max;
+        base.scalars[i] = s->d_scalars;
+        base.tile_lo[i] = (uint32_t)((uint64_t)n_tiles * i / n);
+    }
+    base.tile_lo[n] = n_tiles;
+    std::vector<LightParams> P(n);
+    std::vector<GroupPeers> G(n, base);
+    for (uint32_t i = 0; i < n; i++) {
+        P[i] = propagate_params(gs->scene[i], epsilon);
+        G[i].self = i;
+    }
+    auto ctx = [&](uint32_t i) { return g->ctx[i]; };
+    auto barrier = [&]() -> aicb_status {
+        for (uint32_t i = 1; i < n; i++) {
+            CU(cudaSetDevice(ctx(i)->device));
+            CU(cudaEventRecord(g->light_barrier[i], ctx(i)->stream));
+        }
+        CU(cudaSetDevice(ctx(0)->device));
+        for (uint32_t i = 1; i < n; i++) CU(cudaStreamWaitEvent(ctx(0)->stream, g->light_barrier[i], 0));
+        CU(cudaEventRecord(g->light_barrier[0], ctx(0)->stream));
+        for (uint32_t i = 1; i < n; i++) {
+            CU(cudaSetDevice(ctx(i)->device));
+            CU(cudaStreamWaitEvent(ctx(i)->stream, g->light_barrier[0], 0));
+        }
+        return AICB_OK;
+    };
+    // one step of every member, in member order, on the member's device and stream
+    auto each = [&](auto &&step) -> aicb_status {
+        for (uint32_t i = 0; i < n; i++) {
+            aicb_ctx *c = ctx(i);
+            CU(cudaSetDevice(c->device));
+            const aicb_status r = step(i, c, c->stream, c->num_sms * 8);
+            if (r != AICB_OK) return r;
+        }
+        return AICB_OK;
+    };
+#define GROUP_TRY(call)                          \
+    do {                                         \
+        const aicb_status r__ = (call);          \
+        if (r__ != AICB_OK) return r__;          \
+    } while (0)
+    const bool chains = use_chain_walk();
+    GROUP_TRY(each([&](uint32_t i, aicb_ctx *c, cudaStream_t cs, int blocks) -> aicb_status {
+        CU(cudaEventRecord(c->ev0, cs));
+        CU(cudaMemsetAsync(gs->scene[i]->d_scalars, 0, 16 * 4, cs));
+        k_tile_rebuild<<<blocks, 256, 0, cs>>>(P[i], n_tiles);
+        return AICB_OK;
+    }));
+    const int ROUNDS_PER_SYNC = 8;
+    uint64_t rounds = 0;
+    std::vector<uint32_t> h(16 * n);
+    for (int batch = 0; batch < 100000; batch++) {
+        for (int round = 0; round < ROUNDS_PER_SYNC; round++) {
+            GROUP_TRY(each([&](uint32_t i, aicb_ctx *, cudaStream_t cs, int) -> aicb_status {
+                CU(cudaMemsetAsync(gs->scene[i]->d_scalars, 0, 2 * 4, cs));
+                CU(cudaMemsetAsync(gs->scene[i]->d_scalars + 6, 0, 4 * 4, cs));
+                k_find_max<<<16, 256, 0, cs>>>(P[i], n_tiles);
+                return AICB_OK;
+            }));
+            GROUP_TRY(barrier());   // B1
+            GROUP_TRY(each([&](uint32_t i, aicb_ctx *c, cudaStream_t cs, int blocks) -> aicb_status {
+                k_group_clear_foreign<<<blocks, 256, 0, cs>>>(P[i], G[i], n_tiles);
+                k_group_max<<<1, 32, 0, cs>>>(P[i], G[i]);
+                k_gather<<<blocks, 256, 0, cs>>>(P[i], n_tiles);
+                if (chains) {
+                    k_walk_chains<false><<<c->chain_walk_blocks, 128, 0, cs>>>(P[i], 0, nullptr);
+                    k_compute_overflow<<<blocks, 128, 0, cs>>>(P[i], nullptr);
+                } else {
+                    k_compute<<<blocks, 128, 0, cs>>>(P[i], 0, nullptr);
+                }
+                return AICB_OK;
+            }));
+            GROUP_TRY(barrier());   // B2
+            GROUP_TRY(each([&](uint32_t i, aicb_ctx *, cudaStream_t cs, int blocks) -> aicb_status {
+                k_group_apply<<<blocks, 128, 0, cs>>>(P[i], G[i]);
+                return AICB_OK;
+            }));
+            GROUP_TRY(barrier());   // B3
+            GROUP_TRY(each([&](uint32_t i, aicb_ctx *, cudaStream_t cs, int blocks) -> aicb_status {
+                k_group_guess<<<blocks, 128, 0, cs>>>(P[i], G[i]);
+                return AICB_OK;
+            }));
+            GROUP_TRY(barrier());   // B4
+            GROUP_TRY(each([&](uint32_t i, aicb_ctx *c, cudaStream_t cs, int blocks) -> aicb_status {
+                k_group_broadcast<<<blocks, 128, 0, cs>>>(P[i], G[i]);
+                k_compact_changed<<<blocks, 256, 0, cs>>>(P[i]);
+                if (chains) k_walk_chains<true><<<c->chain_walk_blocks, 128, 0, cs>>>(P[i], 0, nullptr);
+                else k_mark<<<blocks, 128, 0, cs>>>(P[i]);
+                return AICB_OK;
+            }));
+            GROUP_TRY(barrier());   // B5
+            GROUP_TRY(each([&](uint32_t i, aicb_ctx *, cudaStream_t cs, int blocks) -> aicb_status {
+                k_group_merge<<<blocks, 256, 0, cs>>>(P[i], G[i]);
+                return AICB_OK;
+            }));
+        }
+        GROUP_TRY(each([&](uint32_t i, aicb_ctx *, cudaStream_t cs, int) -> aicb_status {
+            CU(cudaMemcpyAsync(&h[16 * i], gs->scene[i]->d_scalars, 16 * 4, cudaMemcpyDeviceToHost, cs));
+            return AICB_OK;
+        }));
+        GROUP_TRY(each([&](uint32_t, aicb_ctx *, cudaStream_t cs, int) -> aicb_status {
+            CU(cudaStreamSynchronize(cs));
+            CU(cudaGetLastError());
+            return AICB_OK;
+        }));
+        rounds += ROUNDS_PER_SYNC;
+        if (h[1] <= P[0].epsilon_priority) break;   // the batch's last round found nothing above epsilon (on any member)
+    }
+    uint64_t total = 0, visits = 0, slowest = 0;
+    uint32_t maxd = 0;
+    GROUP_TRY(each([&](uint32_t, aicb_ctx *c, cudaStream_t cs, int) -> aicb_status {
+        CU(cudaEventRecord(c->ev1, cs));
+        return AICB_OK;
+    }));
+    GROUP_TRY(each([&](uint32_t i, aicb_ctx *c, cudaStream_t, int) -> aicb_status {
+        CU(cudaEventSynchronize(c->ev1));
+        float ms = 0.0f;
+        CU(cudaEventElapsedTime(&ms, c->ev0, c->ev1));
+        aicb_scene *s = gs->scene[i];
+        const uint32_t *hi = &h[16 * i];
+        s->light_stats[0] = hi[3];
+        s->light_stats[1] = (uint64_t)hi[4] | ((uint64_t)hi[5] << 32);
+        s->light_stats[2] = rounds;
+        s->light_stats[3] = (uint64_t)(ms * 1000.0f);
+        total += s->light_stats[0];
+        visits += s->light_stats[1];
+        slowest = s->light_stats[3] > slowest ? s->light_stats[3] : slowest;
+        maxd = hi[2] > maxd ? hi[2] : maxd;
+        return AICB_OK;
+    }));
+#undef GROUP_TRY
+    gs->light_stats[0] = total;
+    gs->light_stats[1] = visits;
+    gs->light_stats[2] = rounds;
+    gs->light_stats[3] = slowest;
+    if (updates_done) *updates_done = total;
+    if (max_diff) *max_diff = (uint8_t)maxd;
+    if (node_visits) *node_visits = visits;
+    return AICB_OK;
+}
+
+// every member's lock, in member order, for the duration of a group call
+struct GroupLock {
+    std::vector<std::unique_lock<std::mutex>> locks;
+    explicit GroupLock(aicb_group_scene *gs) {
+        for (aicb_ctx *c : gs->group->ctx) locks.emplace_back(c->mu);
+    }
+};
+
+// the light state of every replica; LightPhysics::None fails here, before any replica changed
+aicb_status group_ensure_light_state(aicb_group_scene *gs) {
+    for (aicb_scene *s : gs->scene) {
+        CU(cudaSetDevice(s->ctx->device));
+        aicb_status st = ensure_light_state(s);
+        if (st != AICB_OK) return st;
+    }
+    return AICB_OK;
+}
+
+void group_stats_from_member0(aicb_group_scene *gs) {
+    for (int k = 0; k < 4; k++) gs->light_stats[k] = gs->scene[0]->light_stats[k];
+}
+
+}  // namespace
+
+extern "C" {
+
+aicb_status aicb_group_light_fast_evaluate(aicb_group_scene *gs) {
+    if (!gs) return aicb_fail(AICB_ERR_INVALID, "NULL argument");
+    for (aicb_scene *s : gs->scene) {   // every column is computed the same way on every replica
+        aicb_status st = aicb_light_fast_evaluate(s);
+        if (st != AICB_OK) return st;
+    }
+    return AICB_OK;
+}
+
+aicb_status aicb_group_light_evaluate(aicb_group_scene *gs, uint8_t epsilon, uint64_t *updates_done, uint8_t *max_diff,
+                                      uint64_t *node_visits) {
+    if (!gs) return aicb_fail(AICB_ERR_INVALID, "NULL argument");
+    if (gs->scene.size() == 1) {   // one member: the single-scene propagation, without barriers or exchanges
+        aicb_status st = aicb_light_evaluate(gs->scene[0], epsilon, updates_done, max_diff, node_visits);
+        if (st == AICB_OK) group_stats_from_member0(gs);
+        return st;
+    }
+    GroupLock lock(gs);
+    aicb_status st = group_ensure_light_state(gs);
+    if (st != AICB_OK) return st;
+    return group_propagate(gs, epsilon, updates_done, max_diff, node_visits);
+}
+
+aicb_status aicb_group_light_edit_and_propagate(aicb_group_scene *gs, const int32_t (*cubes)[3], const uint16_t *new_ids,
+                                                size_t n_edits, uint8_t epsilon, uint64_t *updates_done, uint8_t *max_diff) {
+    if (!gs || (n_edits && (!cubes || !new_ids))) return aicb_fail(AICB_ERR_INVALID, "NULL argument");
+    if (gs->scene.size() == 1) {
+        aicb_status st = aicb_light_edit_and_propagate(gs->scene[0], cubes, new_ids, n_edits, epsilon, updates_done, max_diff);
+        if (st == AICB_OK) group_stats_from_member0(gs);
+        return st;
+    }
+    GroupLock lock(gs);
+    aicb_status st = group_ensure_light_state(gs);
+    if (st != AICB_OK) return st;
+    // one op list (validated in full before anything changes), applied to every replica and its host mirror
+    std::vector<EditOp> ops;
+    st = edit_ops(gs->scene[0], cubes, new_ids, n_edits, &ops);
+    if (st != AICB_OK) return st;
+    for (size_t m = 1; m < gs->scene.size(); m++) {
+        aicb_scene *s = gs->scene[m];
+        const DeviceScene &ds = s->ds;
+        for (size_t i = 0; i < n_edits; i++) {
+            const size_t idx = ((size_t)(cubes[i][0] - ds.lo[0]) * ds.size[1] + (size_t)(cubes[i][1] - ds.lo[1])) * ds.size[2] +
+                               (size_t)(cubes[i][2] - ds.lo[2]);
+            s->h_ids[idx] = new_ids[i];
+        }
+    }
+    for (aicb_scene *s : gs->scene) {
+        CU(cudaSetDevice(s->ctx->device));
+        st = apply_edit_ops(s, ops);
+        if (st != AICB_OK) return st;
+    }
+    return group_propagate(gs, epsilon, updates_done, max_diff, nullptr);
+}
+
+aicb_status aicb_group_light_download(aicb_group_scene *gs, int member, uint8_t (*out)[4], size_t n_texels) {
+    if (!gs) return aicb_fail(AICB_ERR_INVALID, "NULL argument");
+    if (member < 0 || (size_t)member >= gs->scene.size()) return aicb_fail(AICB_ERR_INVALID, "member out of range");
+    return aicb_light_download(gs->scene[member], out, n_texels);
+}
+
+aicb_status aicb_group_light_stats(const aicb_group_scene *gs, int member, uint64_t out[4]) {
+    if (!gs || !out) return aicb_fail(AICB_ERR_INVALID, "NULL argument");
+    if (member < -1 || member >= (int)gs->scene.size()) return aicb_fail(AICB_ERR_INVALID, "member out of range");
+    const uint64_t *src = member < 0 ? gs->light_stats : gs->scene[member]->light_stats;
+    for (int i = 0; i < 4; i++) out[i] = src[i];
+    return AICB_OK;
+}
+
+}  // extern "C"

@@ -219,6 +219,19 @@ unsafe extern "C" {
                                          light: *const [u8; 4], n: usize) -> aicb_status;
     pub fn aicb_group_render_srgb8(gs: *mut aicb_group_scene, cam: *const aicb_camera, opt: *const aicb_options,
                                    out: *mut [u8; 4], out_len: usize, info: *mut aicb_render_info) -> aicb_status;
+    pub fn aicb_group_scene_update_blocks(gs: *mut aicb_group_scene, indices: *const u16, descs: *const aicb_block_desc,
+                                          n: usize) -> aicb_status;
+    pub fn aicb_group_scene_upload_light(gs: *mut aicb_group_scene, light: *const [u8; 4], n_texels: usize) -> aicb_status;
+    pub fn aicb_group_light_fast_evaluate(gs: *mut aicb_group_scene) -> aicb_status;
+    pub fn aicb_group_light_evaluate(gs: *mut aicb_group_scene, epsilon: u8, updates_done: *mut u64, max_diff: *mut u8,
+                                     chart_node_visits: *mut u64) -> aicb_status;
+    pub fn aicb_group_light_edit_and_propagate(gs: *mut aicb_group_scene, cubes: *const [i32; 3], new_ids: *const u16,
+                                               n_edits: usize, epsilon: u8, updates_done: *mut u64,
+                                               max_diff: *mut u8) -> aicb_status;
+    /// `member` is a position in the group (0..size-1), not a device id.
+    pub fn aicb_group_light_download(gs: *mut aicb_group_scene, member: c_int, out: *mut [u8; 4], n_texels: usize) -> aicb_status;
+    /// `member` -1: the group's totals; else that member's own counters.
+    pub fn aicb_group_light_stats(gs: *const aicb_group_scene, member: c_int, out: *mut [u64; 4]) -> aicb_status;
 
     pub fn aicb_trace_rays(s: *mut aicb_scene, origin_dir: *const [f64; 6], n: usize, opt: *const aicb_options,
                            out_colorbuf: *mut [f32; 4], depth: *mut f64, hit: *mut aicb_hit, steps: *mut u32,

@@ -324,6 +324,25 @@ aicb_status aicb_group_scene_update_cubes(aicb_group_scene *, const int32_t (*cu
 /* == draw_rgba on the whole group: out_len must be fb_width * fb_height. */
 aicb_status aicb_group_render_srgb8(aicb_group_scene *, const aicb_camera *, const aicb_options *,
                                     uint8_t (*out)[4], size_t out_len, aicb_render_info *info_or_null);
+/* aicb_scene_update_blocks / aicb_scene_upload_light on every replica. */
+aicb_status aicb_group_scene_update_blocks(aicb_group_scene *, const uint16_t *indices, const aicb_block_desc *descs, size_t n);
+aicb_status aicb_group_scene_upload_light(aicb_group_scene *, const uint8_t (*light)[4], size_t n_texels);
+/* Light propagation on the group: the aicb_light_* calls of the same names, same semantics and errors.  The relaxation
+ * is sharded by slabs: member i owns an even share of whole queue tiles (1024 cubes, a slab along x) and only the owner
+ * computes and applies its cubes; every applied texel is stored into every replica, so on return every member holds
+ * the same light and aicb_group_render_srgb8 renders it.  Needs peer access with native atomics between every pair of
+ * distinct member devices (AICB_ERR_UNSUPPORTED otherwise; enabled on the first call) and at most 16 members.  Edits
+ * are validated in full before any replica changes.  A group of one member runs the single-scene propagation. */
+aicb_status aicb_group_light_fast_evaluate(aicb_group_scene *);
+aicb_status aicb_group_light_evaluate(aicb_group_scene *, uint8_t epsilon, uint64_t *updates_done, uint8_t *max_diff,
+                                      uint64_t *chart_node_visits_or_null);
+aicb_status aicb_group_light_edit_and_propagate(aicb_group_scene *, const int32_t (*cubes)[3], const uint16_t *new_ids,
+                                                size_t n_edits, uint8_t epsilon, uint64_t *updates_done, uint8_t *max_diff);
+/* member = position in the group (0..size-1), not a device id: the same device may be named twice */
+aicb_status aicb_group_light_download(aicb_group_scene *, int member, uint8_t (*out)[4], size_t n_texels);
+/* As aicb_light_stats for the last group propagation.  member -1: cube updates and chart node visits summed over the
+ * members, rounds, device time of the slowest member; else that member's own counters. */
+aicb_status aicb_group_light_stats(const aicb_group_scene *, int member, uint64_t out[4]);
 
 /* == SpaceRaytracer::trace_ray (sr.rs:113-120) for a batch of explicit rays:
  * origin_dir[i] = {ox,oy,oz,dx,dy,dz}. Output as aicb_render_colorbuf. */
