@@ -16,7 +16,6 @@ aicb_status aicb_cuda_fail(cudaError_t e, const char *what);
         if (e__ != cudaSuccess) return aicb_cuda_fail(e__, #call); \
     } while (0)
 
-struct LightChartNode;  // light_kernel.cuh
 struct LightNodePre;    // light_kernel.cuh
 struct LightChain;      // light_kernel.cuh
 struct LightBlockDev;   // light_kernel.cuh
@@ -70,8 +69,7 @@ struct aicb_ctx {
     void *d_task_aux = nullptr;
     size_t d_task_aux_bytes = 0;
     // light propagation: the static ray chart (space/light/chart), built and uploaded on first use
-    LightChartNode *d_chart = nullptr;
-    LightNodePre *d_chart_pre = nullptr;   // the same chart in depth-first preorder (the lockstep walk)
+    LightNodePre *d_chart_pre = nullptr;   // the chart in depth-first preorder (the overflow walk)
     uint32_t chart_nodes = 0;
     LightChain *d_chains = nullptr;         // the chart as chains, the per-node cube offsets, the Euler tour of the chain tree
     uchar4 *d_node_rel = nullptr;
@@ -109,7 +107,7 @@ struct aicb_scene {
     uint32_t *d_list = nullptr;             // work list of one round (cube indices)
     uint32_t *d_new_light = nullptr;        // computed texels of one round
     uint8_t *d_diff = nullptr;              // difference_priority of one round
-    uint32_t *d_scalars = nullptr;          // [0] list length, [1] max priority, [2] max diff, [3] updates
+    uint32_t *d_scalars = nullptr;          // the propagation's counters (light_kernel.cuh: LightScalar)
     float4 *d_sky_term = nullptr;           // per chart node: the sky light its bundle collects (end_of_ray), for this scene's sky
     uint32_t *d_changed = nullptr;          // list positions whose cube changed by more than one unit this round
     uint32_t *d_tile_max = nullptr;         // per LIGHT_TILE cubes: upper bound of the queued priorities

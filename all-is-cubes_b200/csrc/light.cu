@@ -92,7 +92,7 @@ std::vector<LightChartNode> build_chart() {
     return flat;
 }
 
-// The chart in depth-first preorder, as the lockstep walk (light_kernel.cuh) steps through it: children in Face6
+// The chart in depth-first preorder, as the overflow walk (light_kernel.cuh) steps through it: children in Face6
 // order (the order walk_ray_tree recurses in, updater.rs:500), each node with its depth, its cube relative to the
 // origin, the direction of the step from its parent and the index one past its last descendant.
 std::vector<LightNodePre> build_chart_preorder(const std::vector<LightChartNode> &flat, std::vector<uint32_t> *flat_index = nullptr) {
@@ -204,8 +204,8 @@ const ChainTables &chain_tables_host() {
 }
 
 void free_chart(aicb_ctx *c) {
-    void **ptrs[] = {(void **)&c->d_chart, (void **)&c->d_chart_pre, (void **)&c->d_chains, (void **)&c->d_node_rel,
-                     (void **)&c->d_euler, (void **)&c->d_term_scratch};
+    void **ptrs[] = {(void **)&c->d_chart_pre, (void **)&c->d_chains, (void **)&c->d_node_rel, (void **)&c->d_euler,
+                     (void **)&c->d_term_scratch};
     for (void **p : ptrs) {
         if (*p) cudaFree(*p);
         *p = nullptr;
@@ -237,18 +237,15 @@ aicb_status upload_chart(aicb_ctx *ctx) {
         ctx->chain_walk_blocks = (uint32_t)ctx->num_sms * (uint32_t)per_sm;
         CU(cudaMalloc(&ctx->d_term_scratch, (size_t)ctx->num_sms * CHAIN_WALK_BLOCKS_PER_SM * 4 * LIGHT_WARP_SCRATCH_F4 * sizeof(float4)));
     }
-    std::vector<LightChartNode> chart = build_chart();
     const std::vector<LightNodePre> &pre = chart_preorder_host();
     CU(cudaMalloc(&ctx->d_chart_pre, pre.size() * sizeof(LightNodePre)));
     CU(cudaMemcpy(ctx->d_chart_pre, pre.data(), pre.size() * sizeof(LightNodePre), cudaMemcpyHostToDevice));
-    CU(cudaMalloc(&ctx->d_chart, chart.size() * sizeof(LightChartNode)));
-    CU(cudaMemcpy(ctx->d_chart, chart.data(), chart.size() * sizeof(LightChartNode), cudaMemcpyHostToDevice));
-    ctx->chart_nodes = (uint32_t)chart.size();
+    ctx->chart_nodes = (uint32_t)pre.size();
     return AICB_OK;
 }
 
 aicb_status ensure_chart(aicb_ctx *ctx) {
-    if (ctx->d_chart) return AICB_OK;   // (d_chart is the last allocation of upload_chart)
+    if (ctx->d_chart_pre) return AICB_OK;   // (d_chart_pre is the last allocation of upload_chart)
     const aicb_status st = upload_chart(ctx);
     if (st != AICB_OK) free_chart(ctx);   // a later call starts over instead of leaking the tables that did fit
     return st;
@@ -283,24 +280,22 @@ __global__ void k_find_max(const LightParams P, uint32_t n_tiles) {
     uint32_t m = 0;
     for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < n_tiles; i += gridDim.x * blockDim.x) m = max(m, P.tile_max[i]);
     for (int off = 16; off > 0; off >>= 1) m = max(m, __shfl_down_sync(0xffffffffu, m, off));
-    if ((threadIdx.x & 31) == 0 && m) atomicMax(P.scalars + 1, m);
+    if ((threadIdx.x & 31) == 0 && m) atomicMax(P.scalars + SLOT_PRIORITY, m);
 }
 
-// scalars: [0] cubes gathered this round, [1] highest queued priority this round, [2] largest difference applied
-// (accumulated), [3] cube updates (accumulated), [4..5] chart nodes visited (64-bit, accumulated).
-// A round's kernels read the round's priority and count from device memory, so rounds are queued back to back
-// without a host round trip; a round whose priority is already <= epsilon does nothing.
-// One block per tile: the cubes of a tile reach the list in index order (block-wide scan), so 32 consecutive list
-// entries are neighbours along z — what the lockstep walk wants.
+// One block per tile: the cubes of a tile reach the list in index order (block-wide scan), so consecutive list entries
+// are neighbours.
 __global__ void __launch_bounds__(256) k_gather(const LightParams P, uint32_t n_tiles) {
     __shared__ uint32_t s_part[8], s_max[8], s_base;
-    const uint32_t prio = P.scalars[1];
+    const uint32_t prio = P.scalars[SLOT_PRIORITY];
     if (prio <= P.epsilon_priority) return;
     const uint32_t n_words = (P.volume + 3) / 4;
     const uint32_t lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
     // Thread -> word of the tile.  With a power-of-two z extent the tile is a few whole z-rows, and the threads are
-    // laid out so that 8 consecutive threads (32 cubes: one warp of the lockstep walk) cover a 4 x 8 patch of (y, z)
-    // instead of 32 cubes in a line: neighbours in two directions share more of their chart walk.
+    // laid out so that 8 consecutive threads (32 cubes) cover a 4 x 8 patch of (y, z) instead of 32 cubes in a line.
+    // The layout was chosen for a walk that shared node records between neighbouring cubes.  It stays because it fixes
+    // the list order, the order in which cubes are handed out to the walks and applied: another layout changes the
+    // relaxation's behaviour and its speed.
     uint32_t wl = threadIdx.x;
     {
         const uint32_t nz = (uint32_t)P.scene.size[2];
@@ -338,7 +333,7 @@ __global__ void __launch_bounds__(256) k_gather(const LightParams P, uint32_t n_
         if (threadIdx.x == 0) {
             uint32_t total = 0, m = 0;
             for (int i = 0; i < 8; i++) { const uint32_t c = s_part[i]; s_part[i] = total; total += c; m = max(m, s_max[i]); }
-            s_base = total ? atomicAdd(P.scalars + 0, total) : 0u;
+            s_base = total ? atomicAdd(P.scalars + SLOT_LIST_LEN, total) : 0u;
             P.tile_max[tile] = m;
         }
         __syncthreads();
@@ -353,68 +348,18 @@ __global__ void __launch_bounds__(256) k_gather(const LightParams P, uint32_t n_
     }
 }
 
-// 8 CTAs of 4 warps per SM (64 registers; the records requested ahead spill to L1-resident local memory): the walk is
-// latency bound, and 32 resident warps measured +14 % over the 20 that 94 registers allow (6 / 10 CTAs: +2 % / -30 %).
+// k_compute_overflow: 8 CTAs of 4 warps per SM (64 registers; the records requested ahead spill to L1-resident local
+// memory): the walk is latency bound, and 32 resident warps measured +14 % over the 20 that 94 registers allow (6 / 10
+// CTAs: +2 % / -30 %).
 #ifndef AICB_LIGHT_MIN_BLOCKS
 #define AICB_LIGHT_MIN_BLOCKS 8
 #endif
-// How many consecutive list entries (neighbouring cubes) one warp walks for together.  The walk is a chain of dependent
-// loads per node; a lone warp takes ~1250 cycles per node whatever the number of its lanes that take part.  32 cubes
-// share the most node records, but a round of a few ten thousand cubes then occupies a fraction of the resident
-// warps and lasts as long as its slowest warp (a 32-cube union of ~20 K nodes = 14 ms).  Narrower batches make more,
-// shorter walks: the width is the largest power of two that still yields `P.batches_per_warp` batches per resident warp.
-__device__ __forceinline__ uint32_t batch_width(const LightParams &P, uint32_t n, uint32_t n_warps) {
-    if (P.batch_width) return P.batch_width;
-    uint32_t w = 32;
-    while (w > P.min_batch_width && (uint64_t)n < (uint64_t)n_warps * P.batches_per_warp * w) w >>= 1;
-    return w;
-}
-
-__global__ void __launch_bounds__(128, AICB_LIGHT_MIN_BLOCKS) k_compute(const LightParams P, uint32_t n, const int32_t *explicit_cubes) {
-    __shared__ float s_lut[256];
-    for (int i = threadIdx.x; i < 256; i += blockDim.x) s_lut[i] = P.scene.tables[i];
-    __syncthreads();
-    if (!explicit_cubes) n = P.scalars[0];   // the round's list
-    unsigned long long total_visits = 0;
-    const uint32_t lane = threadIdx.x & 31;
-    const uint32_t n_warps = (gridDim.x * blockDim.x) >> 5;
-    const uint32_t width = batch_width(P, n, n_warps);
-    // batches of `width` consecutive list entries, handed out by a counter: a warp whose cubes see open air walks
-    // ten times the nodes of one whose cubes are enclosed
-    for (;;) {
-        uint32_t batch = 0;
-        if (explicit_cubes) {
-            batch = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;   // (one batch per warp: the grid covers n)
-        } else {
-            if (lane == 0) batch = atomicAdd(P.scalars + 7, 1u);
-            batch = __shfl_sync(0xffffffffu, batch, 0);
-        }
-        const uint32_t base = batch * (explicit_cubes ? 32u : width);
-        if (base >= n) break;
-        const uint32_t i = base + lane;
-        const bool active = i < n && (explicit_cubes || lane < width);
-        int x = 0, y = 0, z = 0;
-        if (active) {
-            if (explicit_cubes) {
-                x = explicit_cubes[3 * i]; y = explicit_cubes[3 * i + 1]; z = explicit_cubes[3 * i + 2];
-            } else {
-                cube_of(P.scene, P.list[i], x, y, z);
-            }
-        }
-        uint32_t visits = 0;
-        const uint32_t nv = compute_light_lockstep<false>(P, s_lut, active, x, y, z, 0, &visits);
-        if (active) P.new_light[i] = nv;
-        total_visits += visits;
-        if (explicit_cubes) break;
-    }
-    for (int off = 16; off > 0; off >>= 1) total_visits += __shfl_down_sync(0xffffffffu, total_visits, off);
-    if (lane == 0 && total_visits) atomicAdd(reinterpret_cast<unsigned long long *>(P.scalars + 4), total_visits);
-}
 
 // compute_light / the dependency re-queue with the chain walk (light_kernel.cuh: compute_light_chains): one warp per
 // cube, cubes handed out by a counter.  k_walk_chains<false> writes new_light for the round's list (or explicit
 // cubes); a cube one of whose chains needs more than LIGHT_CHAIN_K terms goes to the overflow list and is computed by
-// the lockstep walk (k_compute_overflow).  k_walk_chains<true> is k_mark for the entries of `changed`.
+// the overflow walk (k_compute_overflow).  k_walk_chains<true> is the mark walk: the dependency re-queue of
+// apply_light_update (updater.rs:355-360) for the entries of `changed`.
 template <bool MARK>
 __global__ void __launch_bounds__(128, CHAIN_WALK_BLOCKS_PER_SM) k_walk_chains(const LightParams P, uint32_t n, const int32_t *explicit_cubes) {
     __shared__ float s_lut[256];
@@ -424,11 +369,11 @@ __global__ void __launch_bounds__(128, CHAIN_WALK_BLOCKS_PER_SM) k_walk_chains(c
     const uint32_t lane = threadIdx.x & 31, wib = threadIdx.x >> 5;
     ChainShared &sh = s_sh[wib];
     float4 *terms = P.term_scratch + (size_t)(blockIdx.x * 4 + wib) * LIGHT_WARP_SCRATCH_F4;
-    if (!explicit_cubes) n = MARK ? P.scalars[6] : P.scalars[0];
+    if (!explicit_cubes) n = MARK ? P.scalars[SLOT_CHANGED] : P.scalars[SLOT_LIST_LEN];
     unsigned long long total_visits = 0;
     for (;;) {
         uint32_t item = 0;
-        if (lane == 0) item = atomicAdd(P.scalars + (MARK ? 8 : 7), 1u);
+        if (lane == 0) item = atomicAdd(P.scalars + (MARK ? SLOT_MARK_NEXT : SLOT_WALK_NEXT), 1u);
         item = __shfl_sync(0xffffffffu, item, 0);
         if (item >= n) break;
         const uint32_t i = MARK ? P.changed[item] : item;   // position in the round's list
@@ -440,20 +385,20 @@ __global__ void __launch_bounds__(128, CHAIN_WALK_BLOCKS_PER_SM) k_walk_chains(c
         bool overflowed = false;
         const uint32_t nv = compute_light_chains<MARK>(P, s_lut, sh, terms, x, y, z, prio, &visits, &overflowed);
         if (!MARK && lane == 0) {
-            if (overflowed) P.overflow[atomicAdd(P.scalars + 9, 1u)] = i;
+            if (overflowed) P.overflow[atomicAdd(P.scalars + SLOT_OVERFLOW, 1u)] = i;
             else P.new_light[i] = nv;
         }
         total_visits += visits;
     }
-    if (!MARK && lane == 0 && total_visits) atomicAdd(reinterpret_cast<unsigned long long *>(P.scalars + 4), total_visits);
+    if (!MARK && lane == 0 && total_visits) atomicAdd(reinterpret_cast<unsigned long long *>(P.scalars + SLOT_VISITS), total_visits);
 }
 
-// the cubes the chain walk could not hold (scalars[9] entries of `overflow`), by the lockstep walk
+// the overflow walk: the cubes the chain walk could not hold (the SLOT_OVERFLOW entries of `overflow`)
 __global__ void __launch_bounds__(128, AICB_LIGHT_MIN_BLOCKS) k_compute_overflow(const LightParams P, const int32_t *explicit_cubes) {
     __shared__ float s_lut[256];
     for (int i = threadIdx.x; i < 256; i += blockDim.x) s_lut[i] = P.scene.tables[i];
     __syncthreads();
-    const uint32_t n = P.scalars[9];
+    const uint32_t n = P.scalars[SLOT_OVERFLOW];
     const uint32_t lane = threadIdx.x & 31;
     const uint32_t warp = (blockIdx.x * blockDim.x + threadIdx.x) >> 5, n_warps = (gridDim.x * blockDim.x) >> 5;
     unsigned long long total_visits = 0;
@@ -466,27 +411,27 @@ __global__ void __launch_bounds__(128, AICB_LIGHT_MIN_BLOCKS) k_compute_overflow
             else cube_of(P.scene, P.list[i], x, y, z);
         }
         uint32_t visits = 0;
-        const uint32_t nv = compute_light_lockstep<false>(P, s_lut, active, x, y, z, 0, &visits);
+        const uint32_t nv = compute_light_lockstep(P, s_lut, active, x, y, z, &visits);
         if (active) P.new_light[i] = nv;
         total_visits += visits;
     }
     for (int off = 16; off > 0; off >>= 1) total_visits += __shfl_down_sync(0xffffffffu, total_visits, off);
-    if (lane == 0 && total_visits) atomicAdd(reinterpret_cast<unsigned long long *>(P.scalars + 4), total_visits);
+    if (lane == 0 && total_visits) atomicAdd(reinterpret_cast<unsigned long long *>(P.scalars + SLOT_VISITS), total_visits);
 }
 
-// apply_light_update (updater.rs:295-363) minus the dependency re-queue (k_mark)
+// apply_light_update (updater.rs:295-363) minus the dependency re-queue (k_walk_chains<true>)
 __global__ void k_apply(const LightParams P) {
-    const uint32_t n = P.scalars[0];
+    const uint32_t n = P.scalars[SLOT_LIST_LEN];
     for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) {
     const uint32_t idx = P.list[i];
     uint32_t *light = const_cast<uint32_t *>(P.scene.light);
     const uint32_t old = light[idx], nv = P.new_light[i];
     const int d = difference_priority(nv, old);
     P.diff[i] = (uint8_t)d;
-    atomicAdd(P.scalars + 3, 1u);
+    atomicAdd(P.scalars + SLOT_UPDATES, 1u);
     if (d > 0) {
         light[idx] = nv;
-        atomicMax(P.scalars + 2, (uint32_t)d);
+        atomicMax(P.scalars + SLOT_MAX_DIFF, (uint32_t)d);
         int x, y, z;
         cube_of(P.scene, idx, x, y, z);
         const float *lut = P.scene.tables;
@@ -508,11 +453,11 @@ __global__ void k_apply(const LightParams P) {
 }
 
 // apply_light_update re-queues a cube's dependencies only when its packed difference exceeds 1 (updater.rs:355-360).
-// The entries of the round's list that did are compacted (in list order within a block of 256) so that the warps of
-// k_mark walk the chart for 32 cubes that all need it.
+// The entries of the round's list that did are compacted (in list order within a block of 256) so that the mark walk
+// is handed only cubes that need it.
 __global__ void __launch_bounds__(256) k_compact_changed(const LightParams P) {
     __shared__ uint32_t s_part[8], s_base;
-    const uint32_t n = P.scalars[0];
+    const uint32_t n = P.scalars[SLOT_LIST_LEN];
     const uint32_t lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
     for (uint32_t base = blockIdx.x * 256u; base < n; base += gridDim.x * 256u) {
         const uint32_t i = base + threadIdx.x;
@@ -527,33 +472,11 @@ __global__ void __launch_bounds__(256) k_compact_changed(const LightParams P) {
         if (threadIdx.x == 0) {
             uint32_t total = 0;
             for (int k = 0; k < 8; k++) { const uint32_t c = s_part[k]; s_part[k] = total; total += c; }
-            s_base = total ? atomicAdd(P.scalars + 6, total) : 0u;
+            s_base = total ? atomicAdd(P.scalars + SLOT_CHANGED, total) : 0u;
         }
         __syncthreads();
         if (keep) P.changed[s_base + s_part[wid] + inc - 1] = i;
         __syncthreads();
-    }
-}
-
-// the dependency re-queue of apply_light_update (updater.rs:355-360): re-walk the chart, raising the
-// queue priority of every cube whose light was read
-__global__ void __launch_bounds__(128, AICB_LIGHT_MIN_BLOCKS) k_mark(const LightParams P) {
-    const uint32_t n = P.scalars[6];   // entries of the round's list that changed by more than one unit
-    const uint32_t lane = threadIdx.x & 31;
-    const uint32_t n_warps = (gridDim.x * blockDim.x) >> 5;
-    const uint32_t width = batch_width(P, n, n_warps);
-    for (;;) {
-        uint32_t batch = 0;
-        if (lane == 0) batch = atomicAdd(P.scalars + 8, 1u);
-        batch = __shfl_sync(0xffffffffu, batch, 0);
-        const uint32_t base = batch * width;
-        if (base >= n) break;
-        const bool active = base + lane < n && lane < width;
-        const uint32_t i = active ? P.changed[base + lane] : 0u;
-        const int d = active ? (int)P.diff[i] : 0;
-        int x = 0, y = 0, z = 0;
-        if (active) cube_of(P.scene, P.list[i], x, y, z);
-        compute_light_lockstep<true>(P, P.scene.tables, active, x, y, z, (uint32_t)(d / 2 + 1), nullptr);
     }
 }
 
@@ -618,7 +541,6 @@ LightParams make_params(aicb_scene *s) {
     std::memset(&P, 0, sizeof P);
     P.scene = s->ds;
     P.blocks = s->d_light_blocks;
-    P.chart = s->ctx->d_chart;
     P.chart_pre = s->ctx->d_chart_pre;
     P.sky_term = s->d_sky_term;
     P.chains = s->ctx->d_chains;
@@ -627,7 +549,7 @@ LightParams make_params(aicb_scene *s) {
     P.n_chains = s->ctx->n_chains;
     P.n_euler = s->ctx->n_euler;
     P.term_scratch = s->ctx->d_term_scratch;
-    P.overflow = s->d_changed;   // (k_compute's overflow list and k_mark's work list are never live together)
+    P.overflow = s->d_changed;   // (a round's overflow list is consumed before k_compact_changed lists its changed cubes)
     P.chart_nodes = s->ctx->chart_nodes;
     P.tile_max = s->d_tile_max;
     P.changed = s->d_changed;
@@ -687,7 +609,7 @@ aicb_status ensure_light_state(aicb_scene *s) {
         CU(cudaMalloc(&s->d_list, s->volume * 4 + 16));
         CU(cudaMalloc(&s->d_new_light, s->volume * 4 + 16));
         CU(cudaMalloc(&s->d_diff, s->volume + 16));
-        CU(cudaMalloc(&s->d_scalars, 16 * 4));
+        CU(cudaMalloc(&s->d_scalars, LIGHT_SCALARS * 4));
         CU(cudaMalloc(&s->d_tile_max, ((s->volume + LIGHT_TILE - 1) / LIGHT_TILE + 1) * 4));
         CU(cudaMalloc(&s->d_changed, s->volume * 4 + 16));
         s->device_bytes += s->volume * 4;
@@ -696,98 +618,24 @@ aicb_status ensure_light_state(aicb_scene *s) {
     return AICB_OK;
 }
 
-// AICB_LIGHT_WALK=lockstep selects the previous walk (32 cubes per warp in lockstep) for comparisons
-bool use_chain_walk() {
-    const char *e = getenv("AICB_LIGHT_WALK");
-    return !(e && std::strcmp(e, "lockstep") == 0);
-}
-
 // the parameters of a propagation's rounds
 LightParams propagate_params(aicb_scene *s, uint8_t epsilon) {
     LightParams P = make_params(s);
     P.epsilon_priority = (uint32_t)epsilon / 2 + 1;
-    {
-        // Cubes within 16 priority levels of the round's maximum are relaxed together: 3.5x the throughput of
-        // strict level-by-level rounds (few cubes per round leave the GPU idle) for 8 % more updates; the parity
-        // contract (tests/test_gpu_light.py) holds for every band, 0 = one level per round, 255 = all pending cubes.
-        const char *e = getenv("AICB_LIGHT_BAND");
-        P.priority_band = e ? (uint32_t)atoi(e) : 16u;
-        const char *w = getenv("AICB_LIGHT_WIDTH");        // experiments: a fixed batch width (1..32)
-        P.batch_width = w ? (uint32_t)atoi(w) : 0u;
-        const char *b = getenv("AICB_LIGHT_BATCHES_PER_WARP");
-        P.batches_per_warp = b ? (uint32_t)atoi(b) : 2u;
-        const char *m = getenv("AICB_LIGHT_MIN_WIDTH");
-        P.min_batch_width = m ? (uint32_t)atoi(m) : 4u;
-        if (P.batch_width > 32) P.batch_width = 32;
-        if (P.batches_per_warp < 1) P.batches_per_warp = 1;
-        if (P.min_batch_width < 1) P.min_batch_width = 1;
-    }
+    // Cubes within 16 priority levels of the round's maximum are relaxed together: 3.5x the throughput of strict
+    // level-by-level rounds (few cubes per round leave the GPU idle) for 8 % more updates; the parity contract
+    // (tests/test_gpu_light.py) holds for every band, 0 = one level per round, 255 = all pending cubes.
+    const char *e = getenv("AICB_LIGHT_BAND");
+    P.priority_band = e ? (uint32_t)atoi(e) : 16u;
     return P;
 }
 
-// evaluate_light (space.rs:1496-1527): rounds until the highest queued priority is <= from_difference(epsilon)
-aicb_status propagate(aicb_scene *s, uint8_t epsilon, uint64_t *updates_done, uint8_t *max_diff, uint64_t *node_visits) {
-    aicb_ctx *ctx = s->ctx;
-    cudaStream_t st = ctx->stream;
-    const LightParams P = propagate_params(s, epsilon);
-    const int blocks = ctx->num_sms * 8;
-    const int wide = ctx->num_sms * 8;    // 128-thread blocks of the lockstep kernels (one warp per 32 list entries, grid-stride)
-    const uint32_t n_tiles = (uint32_t)((s->volume + LIGHT_TILE - 1) / LIGHT_TILE);
-    uint64_t total = 0, visits = 0, rounds = 0;
-    uint32_t maxd = 0;
-    CU(cudaEventRecord(ctx->ev0, st));
-    CU(cudaMemsetAsync(s->d_scalars, 0, 16 * 4, st));
-    k_tile_rebuild<<<blocks, 256, 0, st>>>(P, n_tiles);   // (fast_evaluate / edits write the priority bytes directly)
-    const int ROUNDS_PER_SYNC = 8;
-    const bool chains = use_chain_walk();
-    for (int batch = 0; batch < 100000; batch++) {
-        for (int round = 0; round < ROUNDS_PER_SYNC; round++) {
-            CU(cudaMemsetAsync(s->d_scalars, 0, 2 * 4, st));   // this round's count and priority
-            CU(cudaMemsetAsync(s->d_scalars + 6, 0, 4 * 4, st));   // ... its count of changed cubes, the two work counters, the overflow count
-            k_find_max<<<16, 256, 0, st>>>(P, n_tiles);
-            k_gather<<<blocks, 256, 0, st>>>(P, n_tiles);
-            if (chains) {
-                k_walk_chains<false><<<ctx->chain_walk_blocks, 128, 0, st>>>(P, 0, nullptr);
-                k_compute_overflow<<<wide, 128, 0, st>>>(P, nullptr);
-            } else {
-                k_compute<<<wide, 128, 0, st>>>(P, 0, nullptr);
-            }
-            k_apply<<<wide, 128, 0, st>>>(P);
-            k_compact_changed<<<blocks, 256, 0, st>>>(P);
-            if (chains) k_walk_chains<true><<<ctx->chain_walk_blocks, 128, 0, st>>>(P, 0, nullptr);
-            else k_mark<<<wide, 128, 0, st>>>(P);
-        }
-        uint32_t h[8];
-        CU(cudaMemcpyAsync(h, s->d_scalars, 8 * 4, cudaMemcpyDeviceToHost, st));
-        CU(cudaStreamSynchronize(st));
-        CU(cudaGetLastError());
-        if (getenv("AICB_LIGHT_TRACE"))
-            fprintf(stderr, "[aicb200 light] batch %d: last round %u cubes at priority %u; %u updates so far\n", batch, h[0], h[1], h[3]);
-        total = h[3];
-        visits = (uint64_t)h[4] | ((uint64_t)h[5] << 32);
-        maxd = h[2];
-        rounds += ROUNDS_PER_SYNC;
-        if (h[1] <= P.epsilon_priority) break;   // the batch's last round found nothing above epsilon
-    }
-    CU(cudaEventRecord(ctx->ev1, st));
-    CU(cudaEventSynchronize(ctx->ev1));
-    float ms = 0.0f;
-    CU(cudaEventElapsedTime(&ms, ctx->ev0, ctx->ev1));
-    s->light_stats[0] = total;
-    s->light_stats[1] = visits;
-    s->light_stats[2] = rounds;
-    s->light_stats[3] = (uint64_t)(ms * 1000.0f);   // device time of the propagation in microseconds
-    if (updates_done) *updates_done = total;
-    if (max_diff) *max_diff = (uint8_t)maxd;
-    if (node_visits) *node_visits = visits;
-    return AICB_OK;
-}
-
-
 // Mutation::set x n (space.rs:1346-1352 -> side_effects_of_set -> modified_cube_needs_update, updater.rs:135-173):
-// validates every edit, then applies them in order to the host mirror and returns what the device has to change.
-// Nothing changes when an edit is invalid.
-aicb_status edit_ops(aicb_scene *s, const int32_t (*cubes)[3], const uint16_t *new_ids, size_t n_edits, std::vector<EditOp> *out) {
+// validates every edit, then applies them in order to the host mirror of every member (the members are replicas) and
+// returns what each member's device has to change.  Nothing changes when an edit is invalid.
+aicb_status edit_ops(const std::vector<aicb_scene *> &members, const int32_t (*cubes)[3], const uint16_t *new_ids,
+                     size_t n_edits, std::vector<EditOp> *out) {
+    const aicb_scene *s = members[0];
     const DeviceScene &ds = s->ds;
     auto index_of = [&](int x, int y, int z, uint32_t *idx) {
         uint32_t dx = (uint32_t)(x - ds.lo[0]), dy = (uint32_t)(y - ds.lo[1]), dz = (uint32_t)(z - ds.lo[2]);
@@ -817,7 +665,7 @@ aicb_status edit_ops(aicb_scene *s, const int32_t (*cubes)[3], const uint16_t *n
         uint32_t idx;
         index_of(cubes[i][0], cubes[i][1], cubes[i][2], &idx);
         if (s->h_ids[idx] == new_ids[i]) continue;  // Mutation::set of the same block changes nothing
-        s->h_ids[idx] = new_ids[i];
+        for (aicb_scene *m : members) m->h_ids[idx] = new_ids[i];
         EditOp &o = op_of(idx);
         o.cell = ds.wide_cells ? (new_ids[i] | ((uint32_t)s->block_kind[new_ids[i]] << 16))
                                : (new_ids[i] | ((uint32_t)s->block_kind[new_ids[i]] << 14));
@@ -859,6 +707,21 @@ aicb_status apply_edit_ops(aicb_scene *s, const std::vector<EditOp> &flat) {
     return AICB_OK;
 }
 
+// the light-side record of a block definition; its flags are also kept on the host (aicb_scene::h_block_light)
+LightBlockDev light_block_of(const aicb_block_desc &b) {
+    LightBlockDev o;
+    std::memset(&o, 0, sizeof o);
+    std::memcpy(o.face_color[0], b.light_color, 16);
+    for (int f = 0; f < 6; f++) std::memcpy(o.face_color[f + 1], b.light_face_colors[f], 16);
+    std::memcpy(o.emission, b.light_emission, 12);
+    uint32_t fl = b.light_opaque_faces & 0x3f;
+    if (fl == 0x3f) fl |= LB_ALL_OPAQUE;
+    if (b.light_visible) fl |= LB_VISIBLE;
+    if (!(b.light_emission[0] == 0.0f && b.light_emission[1] == 0.0f && b.light_emission[2] == 0.0f)) fl |= LB_EMISSIVE;
+    o.flags = fl;
+    return o;
+}
+
 }  // namespace
 
 // ---------------------------------------------------------------------------------------------
@@ -870,17 +733,8 @@ aicb_status aicb_light_scene_upload(aicb_scene *s, const aicb_scene_desc *d) {
     std::vector<LightBlockDev> lb(d->n_blocks);
     s->h_block_light.resize(d->n_blocks);
     for (size_t i = 0; i < d->n_blocks; i++) {
-        const aicb_block_desc &b = d->blocks[i];
-        LightBlockDev &o = lb[i];
-        std::memcpy(o.face_color[0], b.light_color, 16);
-        for (int f = 0; f < 6; f++) std::memcpy(o.face_color[f + 1], b.light_face_colors[f], 16);
-        std::memcpy(o.emission, b.light_emission, 12);
-        uint32_t fl = b.light_opaque_faces & 0x3f;
-        if (fl == 0x3f) fl |= LB_ALL_OPAQUE;
-        if (b.light_visible) fl |= LB_VISIBLE;
-        if (!(b.light_emission[0] == 0.0f && b.light_emission[1] == 0.0f && b.light_emission[2] == 0.0f)) fl |= LB_EMISSIVE;
-        o.flags = fl;
-        s->h_block_light[i] = fl;
+        lb[i] = light_block_of(d->blocks[i]);
+        s->h_block_light[i] = lb[i].flags;
     }
     if (!lb.empty()) {
         CU(cudaMalloc(&s->d_light_blocks, lb.size() * sizeof(LightBlockDev)));
@@ -893,18 +747,8 @@ aicb_status aicb_light_scene_upload(aicb_scene *s, const aicb_scene_desc *d) {
 // the light-side records of replaced block definitions (aicb_scene_update_blocks)
 aicb_status aicb_light_blocks_update(aicb_scene *s, const uint16_t *indices, const aicb_block_desc *descs, size_t n) {
     for (size_t i = 0; i < n; i++) {
-        const aicb_block_desc &b = descs[i];
-        LightBlockDev o;
-        std::memset(&o, 0, sizeof o);
-        std::memcpy(o.face_color[0], b.light_color, 16);
-        for (int f = 0; f < 6; f++) std::memcpy(o.face_color[f + 1], b.light_face_colors[f], 16);
-        std::memcpy(o.emission, b.light_emission, 12);
-        uint32_t fl = b.light_opaque_faces & 0x3f;
-        if (fl == 0x3f) fl |= LB_ALL_OPAQUE;
-        if (b.light_visible) fl |= LB_VISIBLE;
-        if (!(b.light_emission[0] == 0.0f && b.light_emission[1] == 0.0f && b.light_emission[2] == 0.0f)) fl |= LB_EMISSIVE;
-        o.flags = fl;
-        if (indices[i] < s->h_block_light.size()) s->h_block_light[indices[i]] = fl;
+        const LightBlockDev o = light_block_of(descs[i]);
+        if (indices[i] < s->h_block_light.size()) s->h_block_light[indices[i]] = o.flags;
         if (s->d_light_blocks) CU(cudaMemcpy(s->d_light_blocks + indices[i], &o, sizeof o, cudaMemcpyHostToDevice));
     }
     return AICB_OK;
@@ -981,53 +825,22 @@ aicb_status aicb_light_compute(aicb_scene *s, const int32_t (*cubes)[3], size_t 
     int32_t *d_cubes = nullptr;
     CU(cudaMalloc(&d_cubes, n * 12));
     CU(cudaMemcpy(d_cubes, cubes, n * 12, cudaMemcpyHostToDevice));
-    cudaMemsetAsync(s->d_scalars, 0, 16 * 4, s->ctx->stream);
-    if (use_chain_walk()) {
-        k_walk_chains<false><<<s->ctx->chain_walk_blocks, 128, 0, s->ctx->stream>>>(P, (uint32_t)n, d_cubes);
-        k_compute_overflow<<<s->ctx->num_sms * 8, 128, 0, s->ctx->stream>>>(P, d_cubes);
-    } else {
-        k_compute<<<(unsigned)((n + 127) / 128), 128, 0, s->ctx->stream>>>(P, (uint32_t)n, d_cubes);
-    }
-    uint32_t h[16];
+    cudaMemsetAsync(s->d_scalars, 0, LIGHT_SCALARS * 4, s->ctx->stream);
+    k_walk_chains<false><<<s->ctx->chain_walk_blocks, 128, 0, s->ctx->stream>>>(P, (uint32_t)n, d_cubes);
+    k_compute_overflow<<<s->ctx->num_sms * 8, 128, 0, s->ctx->stream>>>(P, d_cubes);
+    uint32_t h[LIGHT_SCALARS];
     cudaError_t e = cudaMemcpyAsync(out, s->d_new_light, n * 4, cudaMemcpyDeviceToHost, s->ctx->stream);
     if (e == cudaSuccess) e = cudaMemcpyAsync(h, s->d_scalars, sizeof h, cudaMemcpyDeviceToHost, s->ctx->stream);
     if (e == cudaSuccess) e = cudaStreamSynchronize(s->ctx->stream);
     if (e == cudaSuccess) {
         s->light_stats[0] = n;
-        s->light_stats[1] = (uint64_t)h[4] | ((uint64_t)h[5] << 32);
-        s->light_stats[2] = h[9];   // cubes that took the lockstep walk (a chain with more terms than its slots)
+        s->light_stats[1] = (uint64_t)h[SLOT_VISITS] | ((uint64_t)h[SLOT_VISITS + 1] << 32);
+        s->light_stats[2] = h[SLOT_OVERFLOW];   // cubes that took the overflow walk (a chain with more terms than its slots)
         s->light_stats[3] = 0;
     }
     cudaFree(d_cubes);
     if (e != cudaSuccess) return aicb_cuda_fail(e, "light compute");
     return AICB_OK;
-}
-
-aicb_status aicb_light_evaluate(aicb_scene *s, uint8_t epsilon, uint64_t *updates_done, uint8_t *max_diff,
-                                uint64_t *node_visits) {
-    if (!s) return aicb_fail(AICB_ERR_INVALID, "NULL argument");
-    std::lock_guard<std::mutex> lock(s->ctx->mu);
-    CU(cudaSetDevice(s->ctx->device));
-    aicb_status st = ensure_light_state(s);
-    if (st != AICB_OK) return st;
-    return propagate(s, epsilon, updates_done, max_diff, node_visits);
-}
-
-// Mutation::set x n (space.rs:1346-1352 -> side_effects_of_set -> modified_cube_needs_update,
-// updater.rs:135-173) applied in order on the host mirror, then evaluate_light(epsilon).
-aicb_status aicb_light_edit_and_propagate(aicb_scene *s, const int32_t (*cubes)[3], const uint16_t *new_ids, size_t n_edits,
-                                          uint8_t epsilon, uint64_t *updates_done, uint8_t *max_diff) {
-    if (!s || (n_edits && (!cubes || !new_ids))) return aicb_fail(AICB_ERR_INVALID, "NULL argument");
-    std::lock_guard<std::mutex> lock(s->ctx->mu);
-    CU(cudaSetDevice(s->ctx->device));
-    aicb_status st = ensure_light_state(s);
-    if (st != AICB_OK) return st;
-    std::vector<EditOp> ops;
-    st = edit_ops(s, cubes, new_ids, n_edits, &ops);
-    if (st != AICB_OK) return st;
-    st = apply_edit_ops(s, ops);
-    if (st != AICB_OK) return st;
-    return propagate(s, epsilon, updates_done, max_diff, nullptr);
 }
 
 aicb_status aicb_light_download(aicb_scene *s, uint8_t (*out)[4], size_t n_texels) {
@@ -1055,7 +868,8 @@ aicb_status aicb_light_stats(const aicb_scene *s, uint64_t out[4]) {
 // Every member holds a full replica of the scene, its light and its queue.  Member i owns the queue tiles
 // [tile_lo[i], tile_lo[i + 1]) (an even split of whole LIGHT_TILE tiles: a slab along x in the Z-major layout, possibly
 // empty); only the owner gathers, computes and applies its cubes.  A round keeps the single-scene round's meaning
-// (propagate()) with barriers (B) between its steps, all stream-ordered through member 0 (no device-side waits):
+// (relax() with one member) with barriers (B) between its steps, all stream-ordered through member 0 (no device-side
+// waits):
 //   find_max over the member's queue            B1
 //   clear the queue outside the member's tiles, round priority := the members' maximum, gather, compute (the member's
 //   full replica is read)                       B2  (no replica is written while a peer may still read it)
@@ -1103,23 +917,23 @@ __global__ void __launch_bounds__(256) k_group_clear_foreign(const LightParams P
 // while it is read here; either value yields the same maximum.
 __global__ void k_group_max(const LightParams P, const GroupPeers G) {
     if (threadIdx.x >= G.n) return;
-    const uint32_t m = *(volatile const uint32_t *)(G.scalars[threadIdx.x] + 1);
-    if (m) atomicMax(P.scalars + 1, m);
+    const uint32_t m = *(volatile const uint32_t *)(G.scalars[threadIdx.x] + SLOT_PRIORITY);
+    if (m) atomicMax(P.scalars + SLOT_PRIORITY, m);
 }
 
 // after B2: apply_light_update (updater.rs:295-363) for the member's own cubes, stored into every replica; the
-// guesses of k_apply are k_group_guess, the dependency re-queue is k_walk_chains<true> / k_mark
+// guesses of k_apply are k_group_guess, the dependency re-queue is k_walk_chains<true>
 __global__ void k_group_apply(const LightParams P, const GroupPeers G) {
-    const uint32_t n = P.scalars[0];
+    const uint32_t n = P.scalars[SLOT_LIST_LEN];
     for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) {
         const uint32_t idx = P.list[i];
         const uint32_t old = P.scene.light[idx], nv = P.new_light[i];
         const int d = difference_priority(nv, old);
         P.diff[i] = (uint8_t)d;
-        atomicAdd(P.scalars + 3, 1u);
+        atomicAdd(P.scalars + SLOT_UPDATES, 1u);
         if (d > 0) {
             for (uint32_t m = 0; m < G.n; m++) G.light[m][idx] = nv;
-            atomicMax(P.scalars + 2, (uint32_t)d);
+            atomicMax(P.scalars + SLOT_MAX_DIFF, (uint32_t)d);
         }
     }
 }
@@ -1127,7 +941,7 @@ __global__ void k_group_apply(const LightParams P, const GroupPeers G) {
 // after B3: PackedLight::guess for the Uninitialized neighbours of the member's changed cubes, as in k_apply, with
 // the CAS on the neighbour's owner's replica (one winner per texel whichever member guesses)
 __global__ void k_group_guess(const LightParams P, const GroupPeers G) {
-    const uint32_t n = P.scalars[0];
+    const uint32_t n = P.scalars[SLOT_LIST_LEN];
     const float *lut = P.scene.tables;
     for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) {
         if (P.diff[i] == 0) continue;
@@ -1153,7 +967,7 @@ __global__ void k_group_guess(const LightParams P, const GroupPeers G) {
 // after B4: the Uninitialized neighbours of the member's changed cubes (every texel a guess may have changed) are
 // copied from their owner's replica into the others.  Several members may store one texel: all store the same value.
 __global__ void k_group_broadcast(const LightParams P, const GroupPeers G) {
-    const uint32_t n = P.scalars[0];
+    const uint32_t n = P.scalars[SLOT_LIST_LEN];
     for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) {
         if (P.diff[i] == 0) continue;
         int x, y, z;
@@ -1225,34 +1039,42 @@ aicb_status group_light_setup(aicb_group *g) {
     return AICB_OK;
 }
 
-// evaluate_light on a group of two or more members (the caller holds every member's lock and has set up the light
-// state of every replica)
-aicb_status group_propagate(aicb_group_scene *gs, uint8_t epsilon, uint64_t *updates_done, uint8_t *max_diff, uint64_t *node_visits) {
-    aicb_group *g = gs->group;
-    const uint32_t n = (uint32_t)gs->scene.size();
-    aicb_status st = group_light_setup(g);
-    if (st != AICB_OK) return st;
-    aicb_scene *s0 = gs->scene[0];
-    const uint32_t n_tiles = (uint32_t)((s0->volume + LIGHT_TILE - 1) / LIGHT_TILE);
-    GroupPeers base;
-    std::memset(&base, 0, sizeof base);
-    base.n = n;
-    for (uint32_t i = 0; i < n; i++) {
-        aicb_scene *s = gs->scene[i];
-        base.light[i] = s->d_light;
-        base.pending[i] = s->d_pending;
-        base.tile_max[i] = s->d_tile_max;
-        base.scalars[i] = s->d_scalars;
-        base.tile_lo[i] = (uint32_t)((uint64_t)n_tiles * i / n);
+// evaluate_light (space.rs:1496-1527) over the members of a propagation: rounds until the highest queued priority is
+// <= from_difference(epsilon).  One member runs the single-scene round; two or more members (the replicas of a device
+// group `g`) run the sharded round above.  The caller holds every member's lock and has set up every member's light
+// state.  Each member's light_stats are its own counters; `group_stats` (may be null) gets the updates and visits
+// summed over the members, the rounds and the slowest member's device time.
+aicb_status relax(const std::vector<aicb_scene *> &members, aicb_group *g, uint8_t epsilon, uint64_t *group_stats,
+                  uint64_t *updates_done, uint8_t *max_diff, uint64_t *node_visits) {
+    const uint32_t n = (uint32_t)members.size();
+    const bool sharded = n > 1;
+    if (sharded) {
+        const aicb_status st = group_light_setup(g);
+        if (st != AICB_OK) return st;
     }
-    base.tile_lo[n] = n_tiles;
+    const uint32_t n_tiles = (uint32_t)((members[0]->volume + LIGHT_TILE - 1) / LIGHT_TILE);
     std::vector<LightParams> P(n);
-    std::vector<GroupPeers> G(n, base);
-    for (uint32_t i = 0; i < n; i++) {
-        P[i] = propagate_params(gs->scene[i], epsilon);
-        G[i].self = i;
+    std::vector<GroupPeers> G(n);
+    if (sharded) {
+        GroupPeers base;
+        std::memset(&base, 0, sizeof base);
+        base.n = n;
+        for (uint32_t i = 0; i < n; i++) {
+            aicb_scene *s = members[i];
+            base.light[i] = s->d_light;
+            base.pending[i] = s->d_pending;
+            base.tile_max[i] = s->d_tile_max;
+            base.scalars[i] = s->d_scalars;
+            base.tile_lo[i] = (uint32_t)((uint64_t)n_tiles * i / n);
+        }
+        base.tile_lo[n] = n_tiles;
+        for (uint32_t i = 0; i < n; i++) {
+            G[i] = base;
+            G[i].self = i;
+        }
     }
-    auto ctx = [&](uint32_t i) { return g->ctx[i]; };
+    for (uint32_t i = 0; i < n; i++) P[i] = propagate_params(members[i], epsilon);
+    auto ctx = [&](uint32_t i) { return members[i]->ctx; };
     auto barrier = [&]() -> aicb_status {
         for (uint32_t i = 1; i < n; i++) {
             CU(cudaSetDevice(ctx(i)->device));
@@ -1277,136 +1099,173 @@ aicb_status group_propagate(aicb_group_scene *gs, uint8_t epsilon, uint64_t *upd
         }
         return AICB_OK;
     };
-#define GROUP_TRY(call)                          \
+#define RELAX_TRY(call)                          \
     do {                                         \
         const aicb_status r__ = (call);          \
         if (r__ != AICB_OK) return r__;          \
     } while (0)
-    const bool chains = use_chain_walk();
-    GROUP_TRY(each([&](uint32_t i, aicb_ctx *c, cudaStream_t cs, int blocks) -> aicb_status {
+    RELAX_TRY(each([&](uint32_t i, aicb_ctx *c, cudaStream_t cs, int blocks) -> aicb_status {
         CU(cudaEventRecord(c->ev0, cs));
-        CU(cudaMemsetAsync(gs->scene[i]->d_scalars, 0, 16 * 4, cs));
-        k_tile_rebuild<<<blocks, 256, 0, cs>>>(P[i], n_tiles);
+        CU(cudaMemsetAsync(members[i]->d_scalars, 0, LIGHT_SCALARS * 4, cs));
+        k_tile_rebuild<<<blocks, 256, 0, cs>>>(P[i], n_tiles);   // (fast_evaluate / edits write the priority bytes directly)
         return AICB_OK;
     }));
     const int ROUNDS_PER_SYNC = 8;
     uint64_t rounds = 0;
-    std::vector<uint32_t> h(16 * n);
+    std::vector<uint32_t> h(LIGHT_SCALARS * n);
     for (int batch = 0; batch < 100000; batch++) {
         for (int round = 0; round < ROUNDS_PER_SYNC; round++) {
-            GROUP_TRY(each([&](uint32_t i, aicb_ctx *, cudaStream_t cs, int) -> aicb_status {
-                CU(cudaMemsetAsync(gs->scene[i]->d_scalars, 0, 2 * 4, cs));
-                CU(cudaMemsetAsync(gs->scene[i]->d_scalars + 6, 0, 4 * 4, cs));
+            RELAX_TRY(each([&](uint32_t i, aicb_ctx *, cudaStream_t cs, int) -> aicb_status {
+                uint32_t *sc = members[i]->d_scalars;
+                CU(cudaMemsetAsync(sc + SLOT_LIST_LEN, 0, (SLOT_PRIORITY - SLOT_LIST_LEN + 1) * 4, cs));
+                CU(cudaMemsetAsync(sc + SLOT_CHANGED, 0, (SLOT_OVERFLOW - SLOT_CHANGED + 1) * 4, cs));
                 k_find_max<<<16, 256, 0, cs>>>(P[i], n_tiles);
                 return AICB_OK;
             }));
-            GROUP_TRY(barrier());   // B1
-            GROUP_TRY(each([&](uint32_t i, aicb_ctx *c, cudaStream_t cs, int blocks) -> aicb_status {
-                k_group_clear_foreign<<<blocks, 256, 0, cs>>>(P[i], G[i], n_tiles);
-                k_group_max<<<1, 32, 0, cs>>>(P[i], G[i]);
-                k_gather<<<blocks, 256, 0, cs>>>(P[i], n_tiles);
-                if (chains) {
-                    k_walk_chains<false><<<c->chain_walk_blocks, 128, 0, cs>>>(P[i], 0, nullptr);
-                    k_compute_overflow<<<blocks, 128, 0, cs>>>(P[i], nullptr);
-                } else {
-                    k_compute<<<blocks, 128, 0, cs>>>(P[i], 0, nullptr);
+            if (sharded) RELAX_TRY(barrier());   // B1
+            RELAX_TRY(each([&](uint32_t i, aicb_ctx *c, cudaStream_t cs, int blocks) -> aicb_status {
+                if (sharded) {
+                    k_group_clear_foreign<<<blocks, 256, 0, cs>>>(P[i], G[i], n_tiles);
+                    k_group_max<<<1, 32, 0, cs>>>(P[i], G[i]);
                 }
+                k_gather<<<blocks, 256, 0, cs>>>(P[i], n_tiles);
+                k_walk_chains<false><<<c->chain_walk_blocks, 128, 0, cs>>>(P[i], 0, nullptr);
+                k_compute_overflow<<<blocks, 128, 0, cs>>>(P[i], nullptr);
+                if (!sharded) k_apply<<<blocks, 128, 0, cs>>>(P[i]);   // apply and guess in one kernel
                 return AICB_OK;
             }));
-            GROUP_TRY(barrier());   // B2
-            GROUP_TRY(each([&](uint32_t i, aicb_ctx *, cudaStream_t cs, int blocks) -> aicb_status {
-                k_group_apply<<<blocks, 128, 0, cs>>>(P[i], G[i]);
-                return AICB_OK;
-            }));
-            GROUP_TRY(barrier());   // B3
-            GROUP_TRY(each([&](uint32_t i, aicb_ctx *, cudaStream_t cs, int blocks) -> aicb_status {
-                k_group_guess<<<blocks, 128, 0, cs>>>(P[i], G[i]);
-                return AICB_OK;
-            }));
-            GROUP_TRY(barrier());   // B4
-            GROUP_TRY(each([&](uint32_t i, aicb_ctx *c, cudaStream_t cs, int blocks) -> aicb_status {
-                k_group_broadcast<<<blocks, 128, 0, cs>>>(P[i], G[i]);
+            if (sharded) {
+                RELAX_TRY(barrier());   // B2
+                RELAX_TRY(each([&](uint32_t i, aicb_ctx *, cudaStream_t cs, int blocks) -> aicb_status {
+                    k_group_apply<<<blocks, 128, 0, cs>>>(P[i], G[i]);
+                    return AICB_OK;
+                }));
+                RELAX_TRY(barrier());   // B3
+                RELAX_TRY(each([&](uint32_t i, aicb_ctx *, cudaStream_t cs, int blocks) -> aicb_status {
+                    k_group_guess<<<blocks, 128, 0, cs>>>(P[i], G[i]);
+                    return AICB_OK;
+                }));
+                RELAX_TRY(barrier());   // B4
+            }
+            RELAX_TRY(each([&](uint32_t i, aicb_ctx *c, cudaStream_t cs, int blocks) -> aicb_status {
+                if (sharded) k_group_broadcast<<<blocks, 128, 0, cs>>>(P[i], G[i]);
                 k_compact_changed<<<blocks, 256, 0, cs>>>(P[i]);
-                if (chains) k_walk_chains<true><<<c->chain_walk_blocks, 128, 0, cs>>>(P[i], 0, nullptr);
-                else k_mark<<<blocks, 128, 0, cs>>>(P[i]);
+                k_walk_chains<true><<<c->chain_walk_blocks, 128, 0, cs>>>(P[i], 0, nullptr);
                 return AICB_OK;
             }));
-            GROUP_TRY(barrier());   // B5
-            GROUP_TRY(each([&](uint32_t i, aicb_ctx *, cudaStream_t cs, int blocks) -> aicb_status {
-                k_group_merge<<<blocks, 256, 0, cs>>>(P[i], G[i]);
-                return AICB_OK;
-            }));
+            if (sharded) {
+                RELAX_TRY(barrier());   // B5
+                RELAX_TRY(each([&](uint32_t i, aicb_ctx *, cudaStream_t cs, int blocks) -> aicb_status {
+                    k_group_merge<<<blocks, 256, 0, cs>>>(P[i], G[i]);
+                    return AICB_OK;
+                }));
+            }
         }
-        GROUP_TRY(each([&](uint32_t i, aicb_ctx *, cudaStream_t cs, int) -> aicb_status {
-            CU(cudaMemcpyAsync(&h[16 * i], gs->scene[i]->d_scalars, 16 * 4, cudaMemcpyDeviceToHost, cs));
+        RELAX_TRY(each([&](uint32_t i, aicb_ctx *, cudaStream_t cs, int) -> aicb_status {
+            CU(cudaMemcpyAsync(&h[LIGHT_SCALARS * i], members[i]->d_scalars, LIGHT_SCALARS * 4, cudaMemcpyDeviceToHost, cs));
             return AICB_OK;
         }));
-        GROUP_TRY(each([&](uint32_t, aicb_ctx *, cudaStream_t cs, int) -> aicb_status {
+        RELAX_TRY(each([&](uint32_t, aicb_ctx *, cudaStream_t cs, int) -> aicb_status {
             CU(cudaStreamSynchronize(cs));
             CU(cudaGetLastError());
             return AICB_OK;
         }));
         rounds += ROUNDS_PER_SYNC;
-        if (h[1] <= P[0].epsilon_priority) break;   // the batch's last round found nothing above epsilon (on any member)
+        // every member's round priority is the members' maximum
+        const uint32_t prio = h[SLOT_PRIORITY];
+        if (getenv("AICB_LIGHT_TRACE")) {
+            uint64_t cubes = 0, updates = 0;
+            for (uint32_t i = 0; i < n; i++) {
+                cubes += h[LIGHT_SCALARS * i + SLOT_LIST_LEN];
+                updates += h[LIGHT_SCALARS * i + SLOT_UPDATES];
+            }
+            fprintf(stderr, "[aicb200 light] batch %d: last round %llu cubes at priority %u; %llu updates so far\n", batch,
+                    (unsigned long long)cubes, prio, (unsigned long long)updates);
+        }
+        if (prio <= P[0].epsilon_priority) break;   // the batch's last round found nothing above epsilon
     }
     uint64_t total = 0, visits = 0, slowest = 0;
     uint32_t maxd = 0;
-    GROUP_TRY(each([&](uint32_t, aicb_ctx *c, cudaStream_t cs, int) -> aicb_status {
+    RELAX_TRY(each([&](uint32_t, aicb_ctx *c, cudaStream_t cs, int) -> aicb_status {
         CU(cudaEventRecord(c->ev1, cs));
         return AICB_OK;
     }));
-    GROUP_TRY(each([&](uint32_t i, aicb_ctx *c, cudaStream_t, int) -> aicb_status {
+    RELAX_TRY(each([&](uint32_t i, aicb_ctx *c, cudaStream_t, int) -> aicb_status {
         CU(cudaEventSynchronize(c->ev1));
         float ms = 0.0f;
         CU(cudaEventElapsedTime(&ms, c->ev0, c->ev1));
-        aicb_scene *s = gs->scene[i];
-        const uint32_t *hi = &h[16 * i];
-        s->light_stats[0] = hi[3];
-        s->light_stats[1] = (uint64_t)hi[4] | ((uint64_t)hi[5] << 32);
+        aicb_scene *s = members[i];
+        const uint32_t *hi = &h[LIGHT_SCALARS * i];
+        s->light_stats[0] = hi[SLOT_UPDATES];
+        s->light_stats[1] = (uint64_t)hi[SLOT_VISITS] | ((uint64_t)hi[SLOT_VISITS + 1] << 32);
         s->light_stats[2] = rounds;
-        s->light_stats[3] = (uint64_t)(ms * 1000.0f);
+        s->light_stats[3] = (uint64_t)(ms * 1000.0f);   // device time of the propagation in microseconds
         total += s->light_stats[0];
         visits += s->light_stats[1];
         slowest = s->light_stats[3] > slowest ? s->light_stats[3] : slowest;
-        maxd = hi[2] > maxd ? hi[2] : maxd;
+        maxd = hi[SLOT_MAX_DIFF] > maxd ? hi[SLOT_MAX_DIFF] : maxd;
         return AICB_OK;
     }));
-#undef GROUP_TRY
-    gs->light_stats[0] = total;
-    gs->light_stats[1] = visits;
-    gs->light_stats[2] = rounds;
-    gs->light_stats[3] = slowest;
+#undef RELAX_TRY
+    if (group_stats) {
+        group_stats[0] = total;
+        group_stats[1] = visits;
+        group_stats[2] = rounds;
+        group_stats[3] = slowest;
+    }
     if (updates_done) *updates_done = total;
     if (max_diff) *max_diff = (uint8_t)maxd;
     if (node_visits) *node_visits = visits;
     return AICB_OK;
 }
 
-// every member's lock, in member order, for the duration of a group call
-struct GroupLock {
+// every member's lock, in member order, for the duration of a call
+struct MemberLock {
     std::vector<std::unique_lock<std::mutex>> locks;
-    explicit GroupLock(aicb_group_scene *gs) {
-        for (aicb_ctx *c : gs->group->ctx) locks.emplace_back(c->mu);
+    explicit MemberLock(const std::vector<aicb_scene *> &members) {
+        for (aicb_scene *s : members) locks.emplace_back(s->ctx->mu);
     }
 };
 
-// the light state of every replica; LightPhysics::None fails here, before any replica changed
-aicb_status group_ensure_light_state(aicb_group_scene *gs) {
-    for (aicb_scene *s : gs->scene) {
+// Mutation::set x n_edits (none for evaluate_light alone) on every member, then evaluate_light(epsilon): a single scene
+// is a propagation of one member.  LightPhysics::None and invalid edits fail before any member changed.
+aicb_status edit_and_relax(const std::vector<aicb_scene *> &members, aicb_group *g, const int32_t (*cubes)[3],
+                           const uint16_t *new_ids, size_t n_edits, uint8_t epsilon, uint64_t *group_stats,
+                           uint64_t *updates_done, uint8_t *max_diff, uint64_t *node_visits) {
+    MemberLock lock(members);
+    for (aicb_scene *s : members) {
         CU(cudaSetDevice(s->ctx->device));
-        aicb_status st = ensure_light_state(s);
+        const aicb_status st = ensure_light_state(s);
         if (st != AICB_OK) return st;
     }
-    return AICB_OK;
-}
-
-void group_stats_from_member0(aicb_group_scene *gs) {
-    for (int k = 0; k < 4; k++) gs->light_stats[k] = gs->scene[0]->light_stats[k];
+    std::vector<EditOp> ops;
+    aicb_status st = edit_ops(members, cubes, new_ids, n_edits, &ops);
+    if (st != AICB_OK) return st;
+    for (aicb_scene *s : members) {
+        CU(cudaSetDevice(s->ctx->device));
+        st = apply_edit_ops(s, ops);
+        if (st != AICB_OK) return st;
+    }
+    return relax(members, g, epsilon, group_stats, updates_done, max_diff, node_visits);
 }
 
 }  // namespace
 
 extern "C" {
+
+aicb_status aicb_light_evaluate(aicb_scene *s, uint8_t epsilon, uint64_t *updates_done, uint8_t *max_diff,
+                                uint64_t *node_visits) {
+    if (!s) return aicb_fail(AICB_ERR_INVALID, "NULL argument");
+    return edit_and_relax({s}, nullptr, nullptr, nullptr, 0, epsilon, nullptr, updates_done, max_diff, node_visits);
+}
+
+// Mutation::set x n (space.rs:1346-1352 -> side_effects_of_set -> modified_cube_needs_update,
+// updater.rs:135-173) applied in order on the host mirror, then evaluate_light(epsilon).
+aicb_status aicb_light_edit_and_propagate(aicb_scene *s, const int32_t (*cubes)[3], const uint16_t *new_ids, size_t n_edits,
+                                          uint8_t epsilon, uint64_t *updates_done, uint8_t *max_diff) {
+    if (!s || (n_edits && (!cubes || !new_ids))) return aicb_fail(AICB_ERR_INVALID, "NULL argument");
+    return edit_and_relax({s}, nullptr, cubes, new_ids, n_edits, epsilon, nullptr, updates_done, max_diff, nullptr);
+}
 
 aicb_status aicb_group_light_fast_evaluate(aicb_group_scene *gs) {
     if (!gs) return aicb_fail(AICB_ERR_INVALID, "NULL argument");
@@ -1420,47 +1279,15 @@ aicb_status aicb_group_light_fast_evaluate(aicb_group_scene *gs) {
 aicb_status aicb_group_light_evaluate(aicb_group_scene *gs, uint8_t epsilon, uint64_t *updates_done, uint8_t *max_diff,
                                       uint64_t *node_visits) {
     if (!gs) return aicb_fail(AICB_ERR_INVALID, "NULL argument");
-    if (gs->scene.size() == 1) {   // one member: the single-scene propagation, without barriers or exchanges
-        aicb_status st = aicb_light_evaluate(gs->scene[0], epsilon, updates_done, max_diff, node_visits);
-        if (st == AICB_OK) group_stats_from_member0(gs);
-        return st;
-    }
-    GroupLock lock(gs);
-    aicb_status st = group_ensure_light_state(gs);
-    if (st != AICB_OK) return st;
-    return group_propagate(gs, epsilon, updates_done, max_diff, node_visits);
+    return edit_and_relax(gs->scene, gs->group, nullptr, nullptr, 0, epsilon, gs->light_stats, updates_done, max_diff,
+                          node_visits);
 }
 
 aicb_status aicb_group_light_edit_and_propagate(aicb_group_scene *gs, const int32_t (*cubes)[3], const uint16_t *new_ids,
                                                 size_t n_edits, uint8_t epsilon, uint64_t *updates_done, uint8_t *max_diff) {
     if (!gs || (n_edits && (!cubes || !new_ids))) return aicb_fail(AICB_ERR_INVALID, "NULL argument");
-    if (gs->scene.size() == 1) {
-        aicb_status st = aicb_light_edit_and_propagate(gs->scene[0], cubes, new_ids, n_edits, epsilon, updates_done, max_diff);
-        if (st == AICB_OK) group_stats_from_member0(gs);
-        return st;
-    }
-    GroupLock lock(gs);
-    aicb_status st = group_ensure_light_state(gs);
-    if (st != AICB_OK) return st;
-    // one op list (validated in full before anything changes), applied to every replica and its host mirror
-    std::vector<EditOp> ops;
-    st = edit_ops(gs->scene[0], cubes, new_ids, n_edits, &ops);
-    if (st != AICB_OK) return st;
-    for (size_t m = 1; m < gs->scene.size(); m++) {
-        aicb_scene *s = gs->scene[m];
-        const DeviceScene &ds = s->ds;
-        for (size_t i = 0; i < n_edits; i++) {
-            const size_t idx = ((size_t)(cubes[i][0] - ds.lo[0]) * ds.size[1] + (size_t)(cubes[i][1] - ds.lo[1])) * ds.size[2] +
-                               (size_t)(cubes[i][2] - ds.lo[2]);
-            s->h_ids[idx] = new_ids[i];
-        }
-    }
-    for (aicb_scene *s : gs->scene) {
-        CU(cudaSetDevice(s->ctx->device));
-        st = apply_edit_ops(s, ops);
-        if (st != AICB_OK) return st;
-    }
-    return group_propagate(gs, epsilon, updates_done, max_diff, nullptr);
+    return edit_and_relax(gs->scene, gs->group, cubes, new_ids, n_edits, epsilon, gs->light_stats, updates_done, max_diff,
+                          nullptr);
 }
 
 aicb_status aicb_group_light_download(aicb_group_scene *gs, int member, uint8_t (*out)[4], size_t n_texels) {

@@ -14,10 +14,10 @@
 // adds up in depth-first order are written to per-chain slots and added afterwards in the Euler tour of the chain
 // tree, which is that order — compute_light on a given field stays bit-identical to the reference.
 //
-// The lockstep walk (compute_light_lockstep) is the previous design, kept for cubes whose walk needs more term slots
-// than a chain holds: one warp steps through the chart in preorder for 32 neighbouring cubes — node record, depth and
-// weights are warp-uniform — and a lane takes part in a node iff its own walk would enter it; a subtree that no lane
-// enters is skipped.  Every lane's f32 additions happen in place, in the reference's order.
+// The overflow walk (compute_light_lockstep) computes the cubes whose walk needs more term slots than a chain holds:
+// one warp steps through the chart in preorder for 32 cubes — node record, depth and weights are warp-uniform — and a
+// lane takes part in a node iff its own walk would enter it; a subtree that no lane enters is skipped.  Every lane's
+// f32 additions happen in place, in the reference's order, so it needs no term slots.
 // The relaxation order differs from the reference's (batch = a priority band), which the reference leaves unspecified
 // (queue.rs:226-246) — parity contract SURVEY §8(a) L4.
 #pragma once
@@ -67,7 +67,7 @@ struct LightChain {
 static_assert(sizeof(LightChain) == 48, "LightChain must be 48 bytes");
 constexpr int LIGHT_MAX_CHAINS = 1056;      // 1043, padded
 constexpr int LIGHT_MAX_BRANCHES = 448;     // 441 chains have children
-constexpr int LIGHT_CHAIN_K = 8;            // entry terms a chain can hold (more: the cube takes the lockstep walk)
+constexpr int LIGHT_CHAIN_K = 8;            // entry terms a chain can hold (more: the cube takes the overflow walk)
 constexpr int LIGHT_CHAIN_SLOTS = LIGHT_CHAIN_K + 1;   // + the term of the pop at the chain's end
 // per-warp scratch in global memory: the term slots, then one light_ahead_cache word per branch slot (rarely used)
 constexpr int LIGHT_WARP_SCRATCH_F4 = LIGHT_MAX_CHAINS * LIGHT_CHAIN_SLOTS + LIGHT_MAX_BRANCHES / 4;
@@ -77,23 +77,35 @@ constexpr int LIGHT_MAX_DEPTH = 224;  // longest chart path is 219 (rays end at 
 
 constexpr uint32_t TX_OPAQUE = 128u << 24, TX_NO_RAYS = 1u << 24, TX_UNINIT = 0u;
 constexpr int PRIO_NEWLY_VISIBLE = 250, PRIO_ESTIMATED = 200;
-#ifndef AICB_LIGHT_GROUP
-#define AICB_LIGHT_GROUP 32
-#endif
-constexpr int LIGHT_GROUP = AICB_LIGHT_GROUP;   // lanes (= neighbouring cubes) that walk the chart together: 4, 8, 16 or 32
 constexpr uint32_t LIGHT_TILE = 1024;   // cubes per queue tile (256 words of pending bytes: one 256-thread block)
+
+// The slots of LightParams::scalars, one propagation's counters in device memory.  A round's kernels read the round's
+// list length and priority from there, so rounds are queued back to back without a host round trip; a round whose
+// priority is already <= epsilon does nothing.  The per-round slots are reset before each round: [LIST_LEN, PRIORITY]
+// and [CHANGED, OVERFLOW]; the others accumulate over the propagation.
+enum LightScalar : uint32_t {
+    SLOT_LIST_LEN = 0,    // cubes gathered this round
+    SLOT_PRIORITY = 1,    // highest queued priority this round
+    SLOT_MAX_DIFF = 2,    // largest difference applied
+    SLOT_UPDATES = 3,     // cube updates
+    SLOT_VISITS = 4,      // chart nodes visited, 64-bit (two slots)
+    SLOT_CHANGED = 6,     // entries of the round's list whose cube changed by more than one unit
+    SLOT_WALK_NEXT = 7,   // the next list entry the compute walk hands out this round
+    SLOT_MARK_NEXT = 8,   // the next `changed` entry the mark walk hands out this round
+    SLOT_OVERFLOW = 9,    // entries of the overflow list this round
+    LIGHT_SCALARS = 16    // slots allocated
+};
 
 struct LightParams {
     aicb::DeviceScene scene;        // cells, light, sky faces, tables (LUT)
     const LightBlockDev *blocks;
-    const LightChartNode *chart;
-    const LightNodePre *chart_pre;
+    const LightNodePre *chart_pre;  // the overflow walk's chart
     const LightChain *chains;       // the chart as chains (breadth-first numbering)
     const uchar4 *node_rel;         // per preorder node: cube relative to the origin (int8 x 3), direction of the step from its parent
     const uint16_t *euler;          // the Euler tour of the chain tree: chain | (0: its entry terms, 1: its pop term) << 15
     uint32_t n_chains, n_euler;
     float4 *term_scratch;           // per resident warp: LIGHT_MAX_CHAINS * LIGHT_CHAIN_SLOTS terms
-    uint32_t *overflow;             // list entries whose walk needs more than LIGHT_CHAIN_K terms in one chain ([9] counts them)
+    uint32_t *overflow;             // list entries whose walk needs more than LIGHT_CHAIN_K terms in one chain
     const float4 *sky_term;         // per preorder node: the sky light its bundle collects at the end of a ray (end_of_ray)
     uint32_t chart_nodes;
     uint32_t *tile_max;             // per LIGHT_TILE cubes: an upper bound of the tile's highest queued priority
@@ -101,15 +113,12 @@ struct LightParams {
     uint32_t *list;
     uint32_t *new_light;
     uint8_t *diff;
-    uint32_t *changed;              // positions in the round's list whose cube changed by more than one unit (k_mark's work)
-    uint32_t *scalars;              // [0] list length, [1] max priority, [2] max diff, [3] updates, [4..5] node visits, [6] changed,
-                                    // [7] / [8] batches handed out by k_compute / k_mark this round, [9] overflow list length
+    uint32_t *changed;              // positions in the round's list whose cube changed by more than one unit (the mark walk's work)
+    uint32_t *scalars;              // LightScalar slots
     uint32_t volume;
     uint32_t max_distance;
     uint32_t priority;              // the round's priority level
     uint32_t epsilon_priority;
-    uint32_t batch_width;       // cubes per warp of the lockstep walk (0: chosen per round from the list length)
-    uint32_t batches_per_warp, min_batch_width;
     uint32_t priority_band;     // cubes whose queued priority is within this many levels of the round's maximum are updated together
 };
 
@@ -215,25 +224,15 @@ __device__ __forceinline__ void end_of_ray(Accum &a, float alpha, float bundle, 
     }
 }
 
-__device__ __forceinline__ unsigned gmask_of_lane() {
-    const unsigned lane = threadIdx.x & 31u;
-    return (LIGHT_GROUP >= 32) ? 0xffffffffu : (((1u << (LIGHT_GROUP & 31)) - 1u) << (lane & ~(unsigned)(LIGHT_GROUP - 1)));
-}
-
 // ---------------------------------------------------------------------------------------------------------------
 // compute_light (updater.rs:368-418) with walk_ray_tree (:427-529) and LightBuffer::traverse (:760-884) for the 32
-// cubes of a warp in lockstep (see the header).  Warp-collective: every lane calls it; `active` = this lane has a
-// cube.  The lockstep unit is a group of LIGHT_GROUP lanes (default: the whole warp).  A group visits the union of
-// its cubes' node sets; with the whole warp 5 of 32 lanes take part in an average node.  Smaller groups have smaller
-// unions, but the groups of a warp then read different node records and cells in the same instruction, and measured
-// on the 128^3 bench scene that costs more than it saves (groups of 4 / 8 / 16 / 32 lanes: 1.31 / 1.44 / 1.61 / 1.87 M
-// cube updates per second): the walk is bound by its memory transactions, not by issue slots.  MARK as in compute_light.  Per-lane state of the walk: `ld`, the depth of the lane's deepest live frame
-// (-1: only the call of the root is pending; -2: the lane does not walk), and its frames (alpha after traverse(),
-// ray_bundle_weight, the children's weight so far, light_ahead_cache) indexed by depth — the depth is warp-uniform,
-// so these local-memory accesses are coalesced.
-template <bool MARK>
-__device__ uint32_t compute_light_lockstep(const LightParams &P, const float *lut, bool active, int ox,
-                                           int oy, int oz, uint32_t mark_priority, uint32_t *visits_out) {
+// cubes of a warp in lockstep (see the header): the overflow walk.  Warp-collective: every lane calls it; `active` =
+// this lane has a cube.  The warp visits the union of its cubes' node sets.  Per-lane state of the walk: `ld`, the
+// depth of the lane's deepest live frame (-1: only the call of the root is pending; -2: the lane does not walk), and
+// its frames (alpha after traverse(), ray_bundle_weight, the children's weight so far, light_ahead_cache) indexed by
+// depth — the depth is warp-uniform, so these local-memory accesses are coalesced.
+__device__ uint32_t compute_light_lockstep(const LightParams &P, const float *lut, bool active, int ox, int oy, int oz,
+                                           uint32_t *visits_out) {
     const DeviceScene &S = P.scene;
     Accum acc = {0.f, 0.f, 0.f, 0.f};
     uint32_t oidx;
@@ -268,18 +267,16 @@ __device__ uint32_t compute_light_lockstep(const LightParams &P, const float *lu
         }
     }
     int ld = (active && !origin_opaque) ? -1 : -2;
-    if (__any_sync(gmask_of_lane(), ld == -1)) {
+    if (__any_sync(0xffffffffu, ld == -1)) {
         float f_alpha[LIGHT_MAX_DEPTH], f_bundle[LIGHT_MAX_DEPTH], f_csum[LIGHT_MAX_DEPTH];
         float f_sky0[LIGHT_MAX_DEPTH], f_sky1[LIGHT_MAX_DEPTH], f_sky2[LIGHT_MAX_DEPTH];
         uint32_t f_ahead[LIGHT_MAX_DEPTH];
         uint8_t f_have[LIGHT_MAX_DEPTH];
         const int max_d2 = (int)(P.max_distance * P.max_distance);
-        const int lane = threadIdx.x & 31;
-        const unsigned gmask = (LIGHT_GROUP >= 32) ? 0xffffffffu : (((1u << (LIGHT_GROUP & 31)) - 1u) << (lane & ~(LIGHT_GROUP - 1)));
         // all children of the frame at depth k are done (updater.rs:518-528): the rest of its bundle ends here
         auto pop_level = [&](int k) {
             if (ld == k) {
-                if (!MARK) end_of_ray(acc, f_alpha[k], fmaxf(f_bundle[k] - f_csum[k], 0.0f), make_float4(f_sky0[k], f_sky1[k], f_sky2[k], 0.f));
+                end_of_ray(acc, f_alpha[k], fmaxf(f_bundle[k] - f_csum[k], 0.0f), make_float4(f_sky0[k], f_sky1[k], f_sky2[k], 0.f));
                 ld = k - 1;
             }
         };
@@ -341,7 +338,7 @@ __device__ uint32_t compute_light_lockstep(const LightParams &P, const float *lu
                 if (bundle > 0.0f) {
                     const int e_x = ox + relx, e_y = oy + rely, e_z = oz + relz;
                     if (too_far || !inb) {
-                        if (!MARK) end_of_ray(acc, e_alpha, bundle, nsky);
+                        end_of_ray(acc, e_alpha, bundle, nsky);
                     } else {
                         // ---- LightBuffer::traverse ----
                         const int dir = (int)(end_dir >> 29);
@@ -367,44 +364,38 @@ __device__ uint32_t compute_light_lockstep(const LightParams &P, const float *lu
                                     int lx = e_x, ly = e_y, lz = e_z;  // hit.adjacent(): the cube the ray came from
                                     const int ax = (e_face - 1) % 3, sgn = (e_face >= 4) ? 1 : -1;
                                     if (ax == 0) lx += sgn; else if (ax == 1) ly += sgn; else lz += sgn;
-                                    if (MARK) mark_dependency(P, lx, ly, lz, mark_priority);
-                                    if (!MARK) {
-                                        const bool e_have_prev = d > 0 && f_have[d - 1] != 0;
-                                        const uint32_t stored = e_have_prev ? f_ahead[d - 1] : light_get(P, lx, ly, lz);
-                                        const float ka = ps_clamped(alpha);
-                                        float lf[3];
-                                        lf[0] = __ldg(&ev->emission[0]) + ps_mul(ps_mul(col[0], lut[stored & 255]), hit_alpha);
-                                        lf[1] = __ldg(&ev->emission[1]) + ps_mul(ps_mul(col[1], lut[(stored >> 8) & 255]), hit_alpha);
-                                        lf[2] = __ldg(&ev->emission[2]) + ps_mul(ps_mul(col[2], lut[(stored >> 16) & 255]), hit_alpha);
-                                        acc.in0 = acc.in0 + ps_mul(ps_mul(lf[0], ka), kw);
-                                        acc.in1 = acc.in1 + ps_mul(ps_mul(lf[1], ka), kw);
-                                        acc.in2 = acc.in2 + ps_mul(ps_mul(lf[2], ka), kw);
-                                    }
+                                    const bool e_have_prev = d > 0 && f_have[d - 1] != 0;
+                                    const uint32_t stored = e_have_prev ? f_ahead[d - 1] : light_get(P, lx, ly, lz);
+                                    const float ka = ps_clamped(alpha);
+                                    float lf[3];
+                                    lf[0] = __ldg(&ev->emission[0]) + ps_mul(ps_mul(col[0], lut[stored & 255]), hit_alpha);
+                                    lf[1] = __ldg(&ev->emission[1]) + ps_mul(ps_mul(col[1], lut[(stored >> 8) & 255]), hit_alpha);
+                                    lf[2] = __ldg(&ev->emission[2]) + ps_mul(ps_mul(col[2], lut[(stored >> 16) & 255]), hit_alpha);
+                                    acc.in0 = acc.in0 + ps_mul(ps_mul(lf[0], ka), kw);
+                                    acc.in1 = acc.in1 + ps_mul(ps_mul(lf[1], ka), kw);
+                                    acc.in2 = acc.in2 + ps_mul(ps_mul(lf[2], ka), kw);
                                     if (hit_opaque_face) alpha = 0.0f; else alpha *= 1.0f - hit_alpha;
                                 }
                                 if (hit_alpha < 1.0f) {
-                                    if (MARK) mark_dependency(P, e_x, e_y, e_z, mark_priority);
-                                    if (!MARK) {
-                                        float sv0 = 0.f, sv1 = 0.f, sv2 = 0.f;
-                                        if (e_face != 0) {
-                                            ahead = S.light[cidx];
-                                            have_ahead = true;
-                                            sv0 = lut[ahead & 255]; sv1 = lut[(ahead >> 8) & 255]; sv2 = lut[(ahead >> 16) & 255];
-                                        }
-                                        const float kh = ps_clamped(hit_alpha), ka = ps_clamped(alpha);
-                                        const float l0 = __ldg(&ev->emission[0]) + ps_mul(sv0, kh);
-                                        const float l1 = __ldg(&ev->emission[1]) + ps_mul(sv1, kh);
-                                        const float l2 = __ldg(&ev->emission[2]) + ps_mul(sv2, kh);
-                                        acc.in0 = acc.in0 + ps_mul(ps_mul(l0, ka), kw);
-                                        acc.in1 = acc.in1 + ps_mul(ps_mul(l1, ka), kw);
-                                        acc.in2 = acc.in2 + ps_mul(ps_mul(l2, ka), kw);
+                                    float sv0 = 0.f, sv1 = 0.f, sv2 = 0.f;
+                                    if (e_face != 0) {
+                                        ahead = S.light[cidx];
+                                        have_ahead = true;
+                                        sv0 = lut[ahead & 255]; sv1 = lut[(ahead >> 8) & 255]; sv2 = lut[(ahead >> 16) & 255];
                                     }
+                                    const float kh = ps_clamped(hit_alpha), ka = ps_clamped(alpha);
+                                    const float l0 = __ldg(&ev->emission[0]) + ps_mul(sv0, kh);
+                                    const float l1 = __ldg(&ev->emission[1]) + ps_mul(sv1, kh);
+                                    const float l2 = __ldg(&ev->emission[2]) + ps_mul(sv2, kh);
+                                    acc.in0 = acc.in0 + ps_mul(ps_mul(l0, ka), kw);
+                                    acc.in1 = acc.in1 + ps_mul(ps_mul(l1, ka), kw);
+                                    acc.in2 = acc.in2 + ps_mul(ps_mul(l2, ka), kw);
                                     alpha *= 1.0f - hit_alpha;
                                 }
                             }
                         }
                         if (!(alpha > 0.0f)) {
-                            if (!MARK) end_of_ray(acc, alpha, bundle, nsky);
+                            end_of_ray(acc, alpha, bundle, nsky);
                         } else {
                             f_alpha[d] = alpha; f_bundle[d] = bundle; f_csum[d] = 0.0f;
                             f_ahead[d] = ahead; f_have[d] = have_ahead ? 1 : 0;
@@ -417,7 +408,7 @@ __device__ uint32_t compute_light_lockstep(const LightParams &P, const float *lu
                 if (d > 0) f_csum[d - 1] += bundle;   // the call returns its bundle weight (updater.rs:514, 528)
             }
             uint32_t next;
-            if (__any_sync(gmask, pushed)) {
+            if (__any_sync(0xffffffffu, pushed)) {
                 top = d;
                 next = n + 1;                    // a child if there is one, else the pops above end the frame
             } else {
@@ -451,7 +442,7 @@ __device__ uint32_t compute_light_lockstep(const LightParams &P, const float *lu
 // compute_light for ONE cube by the whole warp, chain by chain.
 //
 // Phase 1 — the walk.  Ready chains wait in a per-warp queue (shared memory); an idle lane takes one and walks its
-// nodes in order (LightBuffer::traverse, updater.rs:760-884, per node exactly as the lockstep walk does), 32 chains of
+// nodes in order (LightBuffer::traverse, updater.rs:760-884, per node exactly as the overflow walk does), 32 chains of
 // the cube at a time.  A chain that is still alive at its end leaves (alpha, light_ahead_cache) in its branch slot and
 // queues its children.  The walk of a cube visits ~3 K nodes on average; the lockstep walk stepped a warp through the
 // union of 32 cubes' node sets with 5 lanes taking part per node, here every lane steps a node of its own.

@@ -401,7 +401,7 @@ aicb_status aicb_light_download(aicb_scene *, uint8_t (*out)[4], size_t n_texels
  * out[0] cube updates (compute_light calls, updater.rs:368), out[1] chart nodes visited by them, out[2] relaxation
  * rounds queued, out[3] device time of the propagation in microseconds (CUDA events on the context's stream).
  * After aicb_light_compute: out[0] cubes computed, out[1] chart nodes visited, out[2] cubes whose walk needed more
- * term slots than the chain walk holds and took the lockstep walk instead, out[3] 0. */
+ * term slots than the chain walk holds and took the overflow walk instead, out[3] 0. */
 aicb_status aicb_light_stats(const aicb_scene *, uint64_t out[4]);
 
 #ifdef __cplusplus
