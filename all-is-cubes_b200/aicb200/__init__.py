@@ -131,6 +131,12 @@ def load_library() -> C.CDLL:
     lib.aicb_light_compute.argtypes = [C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p]
     lib.aicb_light_evaluate.argtypes = [C.c_void_p, C.c_uint8, C.POINTER(C.c_uint64), C.POINTER(C.c_uint8),
                                         C.POINTER(C.c_uint64)]
+    for prefix in ("aicb_", "aicb_group_"):   # the scene and the group versions take the same arguments
+        getattr(lib, prefix + "light_step").argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_size_t, C.c_uint8,
+                                                        C.c_uint64, C.c_double, C.POINTER(abi.LightUpdates)]
+        getattr(lib, prefix + "light_track_changes").argtypes = [C.c_void_p, C.c_int]
+        getattr(lib, prefix + "light_take_changes").argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_size_t,
+                                                                C.POINTER(C.c_size_t)]
     if lib.aicb_abi_version() != abi.ABI_VERSION:
         raise RuntimeError("libaicb200.so ABI version mismatch")
     _lib = lib
@@ -677,6 +683,59 @@ class SpaceRaytracer:
         lt = np.ascontiguousarray(light, dtype=np.uint8).reshape(-1, 4)
         _check(load_library().aicb_scene_upload_light(self.handle, lt.ctypes.data, lt.shape[0]))
 
+    def light_step(self, cubes=None, block_ids=None, epsilon: int = 0, max_updates: Optional[int] = None,
+                   budget_us: Optional[float] = None) -> dict:
+        """Mutation::set x n, then update_light_from_queue(budget) (updater.rs:181-291): relax until nothing above
+        epsilon is queued, `max_updates` cube updates are done or `budget_us` device microseconds are used up (None:
+        no limit).  -> update_count, queue_count, chart_node_visits, rounds, max_update_difference,
+        max_queue_priority, device_ms."""
+        return _light_step(load_library().aicb_light_step, self.handle, cubes, block_ids, epsilon, max_updates, budget_us)
+
+    def light_track_changes(self, enable: bool = True):
+        """Record the current light as the baseline of light_take_changes (or stop tracking)."""
+        _check(load_library().aicb_light_track_changes(self.handle, 1 if enable else 0))
+
+    def light_take_changes(self):
+        """SpaceChange::CubeLight since the last take: (cubes [n,3] int32, texels [n,4] uint8) in index order."""
+        return _light_take_changes(load_library().aicb_light_take_changes, self.handle)
+
+
+NO_LIMIT = (1 << 64) - 1   # aicb_light_step's max_updates without a limit (UINT64_MAX)
+
+
+def _light_step(fn, handle, cubes, block_ids, epsilon, max_updates, budget_us) -> dict:
+    """aicb_light_step / aicb_group_light_step -> LightUpdatesInfo as a dict."""
+    if cubes is None:
+        c, ids = np.zeros((0, 3), dtype=np.int32), np.zeros(0, dtype=np.uint16)
+    else:
+        c = np.ascontiguousarray(cubes, dtype=np.int32).reshape(-1, 3)
+        ids = np.ascontiguousarray(block_ids, dtype=np.uint16)
+        if ids.shape != (c.shape[0],):
+            raise ValueError("one block id per cube")
+    info = abi.LightUpdates()
+    _check(fn(handle, c.ctypes.data if c.shape[0] else None, ids.ctypes.data if c.shape[0] else None, c.shape[0], epsilon,
+              NO_LIMIT if max_updates is None else int(max_updates), -1.0 if budget_us is None else float(budget_us),
+              C.byref(info)))
+    return {"update_count": int(info.update_count), "queue_count": int(info.queue_count),
+            "chart_node_visits": int(info.chart_node_visits), "rounds": int(info.rounds),
+            "max_update_difference": int(info.max_update_difference),
+            "max_queue_priority": int(info.max_queue_priority), "device_ms": float(info.device_ms)}
+
+
+def _light_take_changes(fn, handle):
+    """The count query, then the take: (cubes [n,3] int32 world coordinates, texels [n,4] uint8)."""
+    n = C.c_size_t(0)
+    while True:
+        _check(fn(handle, None, None, 0, C.byref(n)))
+        cubes = np.zeros((n.value, 3), dtype=np.int32)
+        texels = np.zeros((n.value, 4), dtype=np.uint8)
+        if n.value == 0:
+            return cubes, texels
+        want = n.value
+        _check(fn(handle, cubes.ctypes.data, texels.ctypes.data, want, C.byref(n)))
+        if n.value <= want:    # (a light call between the two may have changed more cubes: ask again)
+            return cubes[:n.value], texels[:n.value]
+
 
 NO_WORLD_TO_SHOW_SRGB8 = (0xBC, 0xBC, 0xBC, 0xFF)   # content/palette.rs:76
 
@@ -808,6 +867,19 @@ class DeviceGroup:
         _check(load_library().aicb_group_light_stats(self.scene, -1 if member is None else member, out))
         return {"cube_updates": int(out[0]), "chart_node_visits": int(out[1]), "rounds": int(out[2]),
                 "device_seconds": int(out[3]) * 1e-6}
+
+    def light_step(self, cubes=None, block_ids=None, epsilon: int = 0, max_updates: Optional[int] = None,
+                   budget_us: Optional[float] = None) -> dict:
+        """SpaceRaytracer.light_step on the group: counts summed over the members, the slowest member's time."""
+        return _light_step(load_library().aicb_group_light_step, self.scene, cubes, block_ids, epsilon, max_updates,
+                           budget_us)
+
+    def light_track_changes(self, enable: bool = True):
+        _check(load_library().aicb_group_light_track_changes(self.scene, 1 if enable else 0))
+
+    def light_take_changes(self):
+        """The changes of member 0's replica (every replica holds the same light)."""
+        return _light_take_changes(load_library().aicb_group_light_take_changes, self.scene)
 
     def draw(self, camera: "Camera", options: "GraphicsOptions") -> "Rendering":
         w, h = camera.data.fb_width, camera.data.fb_height

@@ -108,6 +108,20 @@ class Layer(C.Structure):
     _fields_ = [("scene", C.c_void_p), ("camera", C.POINTER(CameraData)), ("options", C.POINTER(Options))]
 
 
+class LightUpdates(C.Structure):
+    """aicb_light_updates: LightUpdatesInfo (updater.rs:970-984) of one aicb_light_step, plus counters."""
+    _fields_ = [
+        ("update_count", C.c_uint64),
+        ("queue_count", C.c_uint64),
+        ("chart_node_visits", C.c_uint64),
+        ("rounds", C.c_uint32),
+        ("max_update_difference", C.c_uint8),
+        ("max_queue_priority", C.c_uint8),
+        ("_pad", C.c_uint8 * 2),
+        ("device_ms", C.c_float),
+    ]
+
+
 TEXT_ENTERED_SPACE, TEXT_EMPTY, TEXT_INCOMPLETE = -1, -2, -3
 
 EXPORTED_SYMBOLS = [
@@ -169,4 +183,10 @@ EXPORTED_SYMBOLS = [
     "aicb_group_light_edit_and_propagate",
     "aicb_group_light_download",
     "aicb_group_light_stats",
+    "aicb_light_step",
+    "aicb_group_light_step",
+    "aicb_light_track_changes",
+    "aicb_light_take_changes",
+    "aicb_group_light_track_changes",
+    "aicb_group_light_take_changes",
 ]

@@ -111,8 +111,14 @@ struct aicb_scene {
     float4 *d_sky_term = nullptr;           // per chart node: the sky light its bundle collects (end_of_ray), for this scene's sky
     uint32_t *d_changed = nullptr;          // list positions whose cube changed by more than one unit this round
     uint32_t *d_tile_max = nullptr;         // per LIGHT_TILE cubes: upper bound of the queued priorities
+    uint32_t *d_tile_count = nullptr;       // per LIGHT_TILE cubes: a count and its exclusive scan over the tiles (capped
+    uint32_t *d_tile_off = nullptr;         //   rounds of aicb_light_step, aicb_light_take_changes)
     uint32_t light_max_distance = 0;
     uint64_t light_stats[4] = {0, 0, 0, 0};  // last propagation: cube updates, chart node visits, rounds queued, device microseconds
+    double light_us_per_update = 0.1;       // running estimate of device microseconds per cube update (aicb_light_step)
+    uint32_t *d_light_base = nullptr;       // change tracking: the light as of the last take (nullptr: not tracking)
+    uint32_t *d_changes = nullptr;          // records of a take: changes_cap cubes (3 x int32), then changes_cap texels
+    size_t changes_cap = 0;
 };
 
 // One process, several GPUs (group.cu renders, light.cu propagates light): one aicb_ctx per member, the scene

@@ -283,6 +283,35 @@ __global__ void k_find_max(const LightParams P, uint32_t n_tiles) {
     if ((threadIdx.x & 31) == 0 && m) atomicMax(P.scalars + SLOT_PRIORITY, m);
 }
 
+// Thread -> word of the tile in k_gather (which writes it out) and in the capped rounds' kernels.  With a power-of-two
+// z extent the tile is a few whole z-rows, and the threads are laid out so that 8 consecutive threads (32 cubes) cover a
+// 4 x 8 patch of (y, z) instead of 32 cubes in a line.  The layout was chosen for a walk that shared node records between
+// neighbouring cubes.  It stays because it fixes the list order, the order in which cubes are handed out to the walks
+// and applied: another layout changes the relaxation's behaviour and its speed.
+__device__ __forceinline__ uint32_t gather_word_of_thread(const LightParams &P) {
+    uint32_t wl = threadIdx.x;
+    const uint32_t nz = (uint32_t)P.scene.size[2];
+    if (nz >= 8 && nz <= 256 && (nz & (nz - 1)) == 0) {
+        const uint32_t wpr = nz / 4, q = threadIdx.x >> 3, within = threadIdx.x & 7;
+        const uint32_t row_group = q / (wpr / 2), pz = q % (wpr / 2);
+        wl = (row_group * 4 + (within >> 1)) * wpr + pz * 2 + (within & 1);
+    }
+    return wl;
+}
+
+// The bytes of queue word w (value v) in the round's band, as k_gather selects them: bit k set for byte k; *cnt = how
+// many.
+__device__ __forceinline__ uint32_t band_select(const LightParams &P, uint32_t v, uint32_t w, uint32_t prio, uint32_t *cnt) {
+    uint32_t sel = 0, c = 0;
+#pragma unroll
+    for (uint32_t k = 0; k < 4; k++) {
+        const uint32_t p = (v >> (8 * k)) & 255u;
+        if (p > P.epsilon_priority && p + P.priority_band >= prio && w * 4 + k < P.volume) { sel |= 1u << k; c++; }
+    }
+    *cnt = c;
+    return sel;
+}
+
 // One block per tile: the cubes of a tile reach the list in index order (block-wide scan), so consecutive list entries
 // are neighbours.
 __global__ void __launch_bounds__(256) k_gather(const LightParams P, uint32_t n_tiles) {
@@ -291,11 +320,7 @@ __global__ void __launch_bounds__(256) k_gather(const LightParams P, uint32_t n_
     if (prio <= P.epsilon_priority) return;
     const uint32_t n_words = (P.volume + 3) / 4;
     const uint32_t lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
-    // Thread -> word of the tile.  With a power-of-two z extent the tile is a few whole z-rows, and the threads are
-    // laid out so that 8 consecutive threads (32 cubes) cover a 4 x 8 patch of (y, z) instead of 32 cubes in a line.
-    // The layout was chosen for a walk that shared node records between neighbouring cubes.  It stays because it fixes
-    // the list order, the order in which cubes are handed out to the walks and applied: another layout changes the
-    // relaxation's behaviour and its speed.
+    // thread -> word of the tile: gather_word_of_thread, written out here (the inlined helper schedules differently)
     uint32_t wl = threadIdx.x;
     {
         const uint32_t nz = (uint32_t)P.scene.size[2];
@@ -615,6 +640,12 @@ aicb_status ensure_light_state(aicb_scene *s) {
         s->device_bytes += s->volume * 4;
         s->device_bytes += s->volume * 10;
     }
+    if (!s->d_tile_off) {
+        const size_t tiles = (s->volume + LIGHT_TILE - 1) / LIGHT_TILE + 1;
+        CU(cudaMalloc(&s->d_tile_count, tiles * 4));
+        CU(cudaMalloc(&s->d_tile_off, tiles * 4));
+        s->device_bytes += tiles * 8;
+    }
     return AICB_OK;
 }
 
@@ -764,6 +795,10 @@ void aicb_light_scene_free(aicb_scene *s) {
     if (s->d_tile_max) cudaFree(s->d_tile_max);
     if (s->d_changed) cudaFree(s->d_changed);
     if (s->d_sky_term) cudaFree(s->d_sky_term);
+    if (s->d_tile_count) cudaFree(s->d_tile_count);
+    if (s->d_tile_off) cudaFree(s->d_tile_off);
+    if (s->d_light_base) cudaFree(s->d_light_base);
+    if (s->d_changes) cudaFree(s->d_changes);
 }
 
 void aicb_light_ctx_free(aicb_ctx *c) { free_chart(c); }
@@ -1008,6 +1043,243 @@ __global__ void __launch_bounds__(256) k_group_merge(const LightParams P, const 
     }
 }
 
+// ---- capped rounds and the queue report of a step (aicb_light_step) ----
+// A capped round relaxes the same band as an uncapped one but takes only its first `rem` cubes (rem = what is left of
+// the step's cap) in a fixed order: tiles in increasing order, within a tile k_gather's thread -> word and byte order.
+// The members' tiles are consecutive ranges in member order, so that order is global in a group too.
+//   k_band_count   the band's cubes per tile
+//   k_tile_scan    each tile's first rank within the member, and the member's total (SLOT_BAND)
+//   (a group: one more barrier, after which every member's SLOT_BAND is final)
+//   k_band_take    the member's share: clamp(rem - (the band cubes of the members before it), 0, its own); every member
+//                  adds the same total to SLOT_TAKEN
+//   k_gather_capped  the cubes of rank < take, each at its rank in the list; tiles past the cap are left untouched,
+//                  the tile that straddles it keeps its other cubes queued and gets its bound recomputed
+// Compute, apply and mark are the uncapped round's kernels.
+__global__ void __launch_bounds__(256) k_band_count(const LightParams P, uint32_t n_tiles, uint32_t *tile_count) {
+    __shared__ uint32_t s_cnt[8];
+    const uint32_t prio = P.scalars[SLOT_PRIORITY];
+    const uint32_t n_words = (P.volume + 3) / 4;
+    const uint32_t wl = gather_word_of_thread(P);
+    for (uint32_t tile = blockIdx.x; tile < n_tiles; tile += gridDim.x) {
+        const uint32_t tm = P.tile_max[tile];
+        if (prio <= P.epsilon_priority || tm <= P.epsilon_priority || tm + P.priority_band < prio) {   // (block-uniform)
+            if (threadIdx.x == 0) tile_count[tile] = 0;
+            continue;
+        }
+        const uint32_t w = tile * (LIGHT_TILE / 4) + wl;
+        uint32_t cnt;
+        band_select(P, w < n_words ? ((const uint32_t *)P.pending)[w] : 0u, w, prio, &cnt);
+        cnt = __reduce_add_sync(0xffffffffu, cnt);
+        if ((threadIdx.x & 31) == 0) s_cnt[threadIdx.x >> 5] = cnt;
+        __syncthreads();
+        if (threadIdx.x == 0) {
+            uint32_t t = 0;
+            for (int i = 0; i < 8; i++) t += s_cnt[i];
+            tile_count[tile] = t;
+        }
+        __syncthreads();
+    }
+}
+
+// One block of 1024 threads: off[i] = count[0] + ... + count[i - 1]; *total = the sum of all.
+__global__ void __launch_bounds__(1024) k_tile_scan(const uint32_t *count, uint32_t *off, uint32_t n, uint32_t *total) {
+    __shared__ uint32_t s_warp[32];
+    const uint32_t per = (n + blockDim.x - 1) / blockDim.x;
+    const uint32_t lo = min(threadIdx.x * per, n), hi = min(lo + per, n);
+    uint32_t sum = 0;
+    for (uint32_t i = lo; i < hi; i++) sum += count[i];
+    const uint32_t lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
+    uint32_t inc = sum;
+    for (int o = 1; o < 32; o <<= 1) {
+        const uint32_t t = __shfl_up_sync(0xffffffffu, inc, o);
+        if ((int)lane >= o) inc += t;
+    }
+    if (lane == 31) s_warp[wid] = inc;
+    __syncthreads();
+    if (wid == 0) {
+        const uint32_t v = lane < (blockDim.x >> 5) ? s_warp[lane] : 0u;
+        uint32_t vi = v;
+        for (int o = 1; o < 32; o <<= 1) {
+            const uint32_t t = __shfl_up_sync(0xffffffffu, vi, o);
+            if ((int)lane >= o) vi += t;
+        }
+        s_warp[lane] = vi - v;
+        if (lane == 31) *total = vi;
+    }
+    __syncthreads();
+    uint32_t run = s_warp[wid] + inc - sum;
+    for (uint32_t i = lo; i < hi; i++) {
+        off[i] = run;
+        run += count[i];
+    }
+}
+
+// One thread.  Peers' SLOT_BAND are final: they were written before the barrier this kernel follows, and are written
+// again only after the round's later barriers.
+__global__ void k_band_take(const LightParams P, const GroupPeers G, uint32_t cap) {
+    uint32_t before = 0, total = 0;
+    for (uint32_t m = 0; m < G.n; m++) {
+        const uint32_t c = *(volatile const uint32_t *)(G.scalars[m] + SLOT_BAND);
+        if (m < G.self) before += c;
+        total += c;
+    }
+    const uint32_t taken = P.scalars[SLOT_TAKEN];
+    const uint32_t rem = cap > taken ? cap - taken : 0u;
+    P.scalars[SLOT_LIST_LEN] = rem > before ? min(rem - before, P.scalars[SLOT_BAND]) : 0u;
+    P.scalars[SLOT_TAKEN] = taken + min(rem, total);
+}
+
+__global__ void __launch_bounds__(256) k_gather_capped(const LightParams P, uint32_t n_tiles, const uint32_t *tile_off) {
+    __shared__ uint32_t s_part[8], s_max[8];
+    const uint32_t prio = P.scalars[SLOT_PRIORITY];
+    if (prio <= P.epsilon_priority) return;
+    const uint32_t take = P.scalars[SLOT_LIST_LEN];
+    const uint32_t n_words = (P.volume + 3) / 4;
+    const uint32_t lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
+    const uint32_t wl = gather_word_of_thread(P);
+    for (uint32_t tile = blockIdx.x; tile < n_tiles; tile += gridDim.x) {
+        const uint32_t tm = P.tile_max[tile];
+        if (tm <= P.epsilon_priority || tm + P.priority_band < prio) continue;   // (block-uniform)
+        const uint32_t first = tile_off[tile];
+        if (first >= take) continue;   // past the cap (block-uniform)
+        const uint32_t w = tile * (LIGHT_TILE / 4) + wl;
+        uint32_t v = w < n_words ? ((uint32_t *)P.pending)[w] : 0u;
+        uint32_t cnt;
+        const uint32_t sel = band_select(P, v, w, prio, &cnt);
+        uint32_t inc = cnt;
+        for (int off = 1; off < 32; off <<= 1) {
+            const uint32_t t = __shfl_up_sync(0xffffffffu, inc, off);
+            if ((int)lane >= off) inc += t;
+        }
+        if (lane == 31) s_part[wid] = inc;
+        __syncthreads();
+        if (threadIdx.x == 0) {
+            uint32_t total = 0;
+            for (int i = 0; i < 8; i++) { const uint32_t c = s_part[i]; s_part[i] = total; total += c; }
+        }
+        __syncthreads();
+        uint32_t at = first + s_part[wid] + inc - cnt;   // rank of the thread's first band cube
+        uint32_t rest = 0;
+        bool took = false;
+#pragma unroll
+        for (uint32_t k = 0; k < 4; k++) {
+            const uint32_t p = (v >> (8 * k)) & 255u;
+            if ((sel & (1u << k)) && at < take) {
+                P.list[at++] = w * 4 + k;
+                v &= ~(255u << (8 * k));
+                took = true;
+            } else {
+                rest = max(rest, p);
+            }
+        }
+        if (took) ((uint32_t *)P.pending)[w] = v;
+        rest = __reduce_max_sync(0xffffffffu, rest);
+        if (lane == 0) s_max[wid] = rest;
+        __syncthreads();
+        if (threadIdx.x == 0) {
+            uint32_t m = 0;
+            for (int i = 0; i < 8; i++) m = max(m, s_max[i]);
+            P.tile_max[tile] = m;
+        }
+        __syncthreads();
+    }
+}
+
+// The queue report of a step: queued cubes and their highest priority in the member's own tiles (after the merge, they
+// hold the member's share of the queue), reading only the tiles whose bound is above 0.
+__global__ void __launch_bounds__(256) k_queue_report(const LightParams P, const GroupPeers G) {
+    const uint32_t lo = G.tile_lo[G.self], hi = G.tile_lo[G.self + 1];
+    const uint32_t n_words = (P.volume + 3) / 4;
+    for (uint32_t tile = lo + blockIdx.x; tile < hi; tile += gridDim.x) {
+        if (P.tile_max[tile] == 0) continue;   // (block-uniform)
+        const uint32_t w = tile * (LIGHT_TILE / 4) + threadIdx.x;
+        const uint32_t v = w < n_words ? ((const uint32_t *)P.pending)[w] : 0u;
+        uint32_t cnt = 0, m = 0;
+#pragma unroll
+        for (uint32_t k = 0; k < 4; k++) {
+            const uint32_t p = (v >> (8 * k)) & 255u;
+            cnt += p ? 1u : 0u;
+            m = max(m, p);
+        }
+        cnt = __reduce_add_sync(0xffffffffu, cnt);
+        m = __reduce_max_sync(0xffffffffu, m);
+        if ((threadIdx.x & 31) == 0 && cnt) {
+            atomicAdd(P.scalars + SLOT_QUEUED, cnt);
+            atomicMax(P.scalars + SLOT_QUEUE_MAX, m);
+        }
+    }
+}
+
+// ---- change tracking (aicb_light_take_changes): texels that differ from the baseline, per tile of LIGHT_TILE cubes
+// (one block of 256 threads, 4 consecutive cubes per thread, so a tile's cubes are in index order) ----
+__device__ __forceinline__ uint32_t diff_mask(const uint32_t *light, const uint32_t *base, uint32_t volume, uint32_t i0) {
+    uint32_t mask = 0;
+#pragma unroll
+    for (uint32_t k = 0; k < 4; k++)
+        if (i0 + k < volume && light[i0 + k] != base[i0 + k]) mask |= 1u << k;
+    return mask;
+}
+
+__global__ void __launch_bounds__(256) k_diff_count(const uint32_t *light, const uint32_t *base, uint32_t volume,
+                                                    uint32_t n_tiles, uint32_t *tile_count) {
+    __shared__ uint32_t s_cnt[8];
+    for (uint32_t tile = blockIdx.x; tile < n_tiles; tile += gridDim.x) {
+        uint32_t cnt = __popc(diff_mask(light, base, volume, tile * LIGHT_TILE + 4 * threadIdx.x));
+        cnt = __reduce_add_sync(0xffffffffu, cnt);
+        if ((threadIdx.x & 31) == 0) s_cnt[threadIdx.x >> 5] = cnt;
+        __syncthreads();
+        if (threadIdx.x == 0) {
+            uint32_t t = 0;
+            for (int i = 0; i < 8; i++) t += s_cnt[i];
+            tile_count[tile] = t;
+        }
+        __syncthreads();
+    }
+}
+
+// the records of the changed texels at their rank (tile_off = the scan of k_diff_count's counts), and the baseline of
+// those cubes moved to the current light
+__global__ void __launch_bounds__(256) k_diff_take(const DeviceScene S, uint32_t *base, uint32_t n_tiles,
+                                                   const uint32_t *tile_count, const uint32_t *tile_off,
+                                                   int32_t *cubes, uint32_t *texels) {
+    __shared__ uint32_t s_part[8];
+    const uint32_t volume = (uint32_t)S.size[0] * (uint32_t)S.size[1] * (uint32_t)S.size[2];
+    const uint32_t lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
+    for (uint32_t tile = blockIdx.x; tile < n_tiles; tile += gridDim.x) {
+        if (tile_count[tile] == 0) continue;   // (block-uniform)
+        const uint32_t i0 = tile * LIGHT_TILE + 4 * threadIdx.x;
+        const uint32_t mask = diff_mask(S.light, base, volume, i0);
+        const uint32_t cnt = __popc(mask);
+        uint32_t inc = cnt;
+        for (int off = 1; off < 32; off <<= 1) {
+            const uint32_t t = __shfl_up_sync(0xffffffffu, inc, off);
+            if ((int)lane >= off) inc += t;
+        }
+        if (lane == 31) s_part[wid] = inc;
+        __syncthreads();
+        if (threadIdx.x == 0) {
+            uint32_t total = 0;
+            for (int i = 0; i < 8; i++) { const uint32_t c = s_part[i]; s_part[i] = total; total += c; }
+        }
+        __syncthreads();
+        uint32_t at = tile_off[tile] + s_part[wid] + inc - cnt;
+#pragma unroll
+        for (uint32_t k = 0; k < 4; k++) {
+            if (!(mask & (1u << k))) continue;
+            const uint32_t idx = i0 + k, t = S.light[idx];
+            int x, y, z;
+            cube_of(S, idx, x, y, z);
+            cubes[3 * at] = x;
+            cubes[3 * at + 1] = y;
+            cubes[3 * at + 2] = z;
+            texels[at] = t;
+            base[idx] = t;
+            at++;
+        }
+        __syncthreads();
+    }
+}
+
 // Peer access between every pair of distinct member devices, with native atomics (k_group_guess); members on one
 // device need neither.  Once per group.
 aicb_status group_light_setup(aicb_group *g) {
@@ -1044,8 +1316,14 @@ aicb_status group_light_setup(aicb_group *g) {
 // group `g`) run the sharded round above.  The caller holds every member's lock and has set up every member's light
 // state.  Each member's light_stats are its own counters; `group_stats` (may be null) gets the updates and visits
 // summed over the members, the rounds and the slowest member's device time.
+// `step` (aicb_light_step; null for evaluate_light) adds the queue report and, with a cap below UINT64_MAX, runs capped
+// rounds that stop once the step has taken `cap` cubes; a cap of 0 runs no round.
+struct StepArgs {
+    uint64_t cap;
+    aicb_light_updates *out;   // filled on success (not null)
+};
 aicb_status relax(const std::vector<aicb_scene *> &members, aicb_group *g, uint8_t epsilon, uint64_t *group_stats,
-                  uint64_t *updates_done, uint8_t *max_diff, uint64_t *node_visits) {
+                  uint64_t *updates_done, uint8_t *max_diff, uint64_t *node_visits, const StepArgs *step = nullptr) {
     const uint32_t n = (uint32_t)members.size();
     const bool sharded = n > 1;
     if (sharded) {
@@ -1054,8 +1332,8 @@ aicb_status relax(const std::vector<aicb_scene *> &members, aicb_group *g, uint8
     }
     const uint32_t n_tiles = (uint32_t)((members[0]->volume + LIGHT_TILE - 1) / LIGHT_TILE);
     std::vector<LightParams> P(n);
-    std::vector<GroupPeers> G(n);
-    if (sharded) {
+    std::vector<GroupPeers> G(n);   // (a single member's: its own tiles, for the step's kernels)
+    {
         GroupPeers base;
         std::memset(&base, 0, sizeof base);
         base.n = n;
@@ -1074,6 +1352,8 @@ aicb_status relax(const std::vector<aicb_scene *> &members, aicb_group *g, uint8
         }
     }
     for (uint32_t i = 0; i < n; i++) P[i] = propagate_params(members[i], epsilon);
+    const bool capped = step && step->cap != UINT64_MAX;
+    const uint32_t cap = capped ? (uint32_t)(step->cap < 0xffffffffull ? step->cap : 0xffffffffull) : 0u;
     auto ctx = [&](uint32_t i) { return members[i]->ctx; };
     auto barrier = [&]() -> aicb_status {
         for (uint32_t i = 1; i < n; i++) {
@@ -1113,7 +1393,7 @@ aicb_status relax(const std::vector<aicb_scene *> &members, aicb_group *g, uint8
     const int ROUNDS_PER_SYNC = 8;
     uint64_t rounds = 0;
     std::vector<uint32_t> h(LIGHT_SCALARS * n);
-    for (int batch = 0; batch < 100000; batch++) {
+    for (int batch = 0; batch < 100000 && !(capped && cap == 0); batch++) {
         for (int round = 0; round < ROUNDS_PER_SYNC; round++) {
             RELAX_TRY(each([&](uint32_t i, aicb_ctx *, cudaStream_t cs, int) -> aicb_status {
                 uint32_t *sc = members[i]->d_scalars;
@@ -1123,12 +1403,30 @@ aicb_status relax(const std::vector<aicb_scene *> &members, aicb_group *g, uint8
                 return AICB_OK;
             }));
             if (sharded) RELAX_TRY(barrier());   // B1
+            if (capped) {
+                RELAX_TRY(each([&](uint32_t i, aicb_ctx *, cudaStream_t cs, int blocks) -> aicb_status {
+                    if (sharded) {
+                        k_group_clear_foreign<<<blocks, 256, 0, cs>>>(P[i], G[i], n_tiles);
+                        k_group_max<<<1, 32, 0, cs>>>(P[i], G[i]);
+                    }
+                    aicb_scene *s = members[i];
+                    k_band_count<<<blocks, 256, 0, cs>>>(P[i], n_tiles, s->d_tile_count);
+                    k_tile_scan<<<1, 1024, 0, cs>>>(s->d_tile_count, s->d_tile_off, n_tiles, s->d_scalars + SLOT_BAND);
+                    return AICB_OK;
+                }));
+                if (sharded) RELAX_TRY(barrier());   // every member's SLOT_BAND is final
+            }
             RELAX_TRY(each([&](uint32_t i, aicb_ctx *c, cudaStream_t cs, int blocks) -> aicb_status {
-                if (sharded) {
-                    k_group_clear_foreign<<<blocks, 256, 0, cs>>>(P[i], G[i], n_tiles);
-                    k_group_max<<<1, 32, 0, cs>>>(P[i], G[i]);
+                if (capped) {
+                    k_band_take<<<1, 1, 0, cs>>>(P[i], G[i], cap);
+                    k_gather_capped<<<blocks, 256, 0, cs>>>(P[i], n_tiles, members[i]->d_tile_off);
+                } else {
+                    if (sharded) {
+                        k_group_clear_foreign<<<blocks, 256, 0, cs>>>(P[i], G[i], n_tiles);
+                        k_group_max<<<1, 32, 0, cs>>>(P[i], G[i]);
+                    }
+                    k_gather<<<blocks, 256, 0, cs>>>(P[i], n_tiles);
                 }
-                k_gather<<<blocks, 256, 0, cs>>>(P[i], n_tiles);
                 k_walk_chains<false><<<c->chain_walk_blocks, 128, 0, cs>>>(P[i], 0, nullptr);
                 k_compute_overflow<<<blocks, 128, 0, cs>>>(P[i], nullptr);
                 if (!sharded) k_apply<<<blocks, 128, 0, cs>>>(P[i]);   // apply and guess in one kernel
@@ -1183,17 +1481,28 @@ aicb_status relax(const std::vector<aicb_scene *> &members, aicb_group *g, uint8
                     (unsigned long long)cubes, prio, (unsigned long long)updates);
         }
         if (prio <= P[0].epsilon_priority) break;   // the batch's last round found nothing above epsilon
+        if (capped && h[SLOT_TAKEN] >= cap) break;   // the step's cap is used up
     }
-    uint64_t total = 0, visits = 0, slowest = 0;
-    uint32_t maxd = 0;
+    if (step) {
+        RELAX_TRY(each([&](uint32_t i, aicb_ctx *, cudaStream_t cs, int blocks) -> aicb_status {
+            k_queue_report<<<blocks, 256, 0, cs>>>(P[i], G[i]);
+            CU(cudaMemcpyAsync(&h[LIGHT_SCALARS * i], members[i]->d_scalars, LIGHT_SCALARS * 4, cudaMemcpyDeviceToHost, cs));
+            return AICB_OK;
+        }));
+    }
+    uint64_t total = 0, visits = 0, slowest = 0, queued = 0;
+    uint32_t maxd = 0, queue_max = 0;
+    float slowest_ms = 0.0f;
     RELAX_TRY(each([&](uint32_t, aicb_ctx *c, cudaStream_t cs, int) -> aicb_status {
         CU(cudaEventRecord(c->ev1, cs));
         return AICB_OK;
     }));
     RELAX_TRY(each([&](uint32_t i, aicb_ctx *c, cudaStream_t, int) -> aicb_status {
         CU(cudaEventSynchronize(c->ev1));
+        CU(cudaGetLastError());
         float ms = 0.0f;
         CU(cudaEventElapsedTime(&ms, c->ev0, c->ev1));
+        slowest_ms = ms > slowest_ms ? ms : slowest_ms;
         aicb_scene *s = members[i];
         const uint32_t *hi = &h[LIGHT_SCALARS * i];
         s->light_stats[0] = hi[SLOT_UPDATES];
@@ -1204,6 +1513,8 @@ aicb_status relax(const std::vector<aicb_scene *> &members, aicb_group *g, uint8
         visits += s->light_stats[1];
         slowest = s->light_stats[3] > slowest ? s->light_stats[3] : slowest;
         maxd = hi[SLOT_MAX_DIFF] > maxd ? hi[SLOT_MAX_DIFF] : maxd;
+        queued += hi[SLOT_QUEUED];
+        queue_max = hi[SLOT_QUEUE_MAX] > queue_max ? hi[SLOT_QUEUE_MAX] : queue_max;
         return AICB_OK;
     }));
 #undef RELAX_TRY
@@ -1216,6 +1527,17 @@ aicb_status relax(const std::vector<aicb_scene *> &members, aicb_group *g, uint8
     if (updates_done) *updates_done = total;
     if (max_diff) *max_diff = (uint8_t)maxd;
     if (node_visits) *node_visits = visits;
+    if (step) {
+        aicb_light_updates &o = *step->out;
+        std::memset(&o, 0, sizeof o);
+        o.update_count = total;
+        o.queue_count = queued;
+        o.chart_node_visits = visits;
+        o.rounds = (uint32_t)rounds;
+        o.max_update_difference = (uint8_t)maxd;
+        o.max_queue_priority = (uint8_t)queue_max;
+        o.device_ms = slowest_ms;
+    }
     return AICB_OK;
 }
 
@@ -1229,9 +1551,14 @@ struct MemberLock {
 
 // Mutation::set x n_edits (none for evaluate_light alone) on every member, then evaluate_light(epsilon): a single scene
 // is a propagation of one member.  LightPhysics::None and invalid edits fail before any member changed.
+// A step (max_updates not null: aicb_light_step) turns its time budget into an update cap with members[0]'s estimate of
+// device microseconds per update, as update_light_from_queue turns the time left into a cost budget
+// (updater.rs:197-203, 270-278), and refines the estimate afterwards.
 aicb_status edit_and_relax(const std::vector<aicb_scene *> &members, aicb_group *g, const int32_t (*cubes)[3],
                            const uint16_t *new_ids, size_t n_edits, uint8_t epsilon, uint64_t *group_stats,
-                           uint64_t *updates_done, uint8_t *max_diff, uint64_t *node_visits) {
+                           uint64_t *updates_done, uint8_t *max_diff, uint64_t *node_visits,
+                           const uint64_t *max_updates = nullptr, double budget_us = -1.0, aicb_light_updates *out = nullptr) {
+    if (budget_us != budget_us) return aicb_fail(AICB_ERR_INVALID, "budget_us is NaN");
     MemberLock lock(members);
     for (aicb_scene *s : members) {
         CU(cudaSetDevice(s->ctx->device));
@@ -1246,7 +1573,92 @@ aicb_status edit_and_relax(const std::vector<aicb_scene *> &members, aicb_group 
         st = apply_edit_ops(s, ops);
         if (st != AICB_OK) return st;
     }
-    return relax(members, g, epsilon, group_stats, updates_done, max_diff, node_visits);
+    if (!max_updates) return relax(members, g, epsilon, group_stats, updates_done, max_diff, node_visits);
+    aicb_scene *lead = members[0];
+    uint64_t cap = *max_updates;
+    if (budget_us >= 0.0) {
+        const double c = std::floor(budget_us / lead->light_us_per_update);
+        uint64_t by_time = c >= 1.8e19 ? UINT64_MAX - 1 : (uint64_t)c;
+        if (budget_us > 0.0 && by_time == 0) by_time = 1;
+        cap = by_time < cap ? by_time : cap;
+    }
+    aicb_light_updates info;
+    const StepArgs step{cap, out ? out : &info};
+    st = relax(members, g, epsilon, group_stats, updates_done, max_diff, node_visits, &step);
+    if (st != AICB_OK) return st;
+    // device microseconds per cube update, a running average with weight 1/8 per step
+    const aicb_light_updates &r = *step.out;
+    if (r.update_count > 0) {
+        const double us = (double)r.device_ms * 1000.0 / (double)r.update_count;
+        lead->light_us_per_update += (us - lead->light_us_per_update) / 8.0;
+    }
+    return AICB_OK;
+}
+
+// change tracking on one scene (a group: member 0); the caller holds the scene's lock
+aicb_status track_changes(aicb_scene *s, int enable) {
+    CU(cudaSetDevice(s->ctx->device));
+    if (!enable) {
+        if (s->d_light_base) {
+            CU(cudaStreamSynchronize(s->ctx->stream));
+            cudaFree(s->d_light_base);
+            s->d_light_base = nullptr;
+            s->device_bytes -= s->volume * 4;
+        }
+        if (s->d_changes) {
+            cudaFree(s->d_changes);
+            s->d_changes = nullptr;
+            s->device_bytes -= s->changes_cap * 16;
+            s->changes_cap = 0;
+        }
+        return AICB_OK;
+    }
+    const aicb_status st = ensure_light_state(s);
+    if (st != AICB_OK) return st;
+    if (!s->d_light_base) {
+        CU(cudaMalloc(&s->d_light_base, s->volume * 4 + 16));
+        s->device_bytes += s->volume * 4;
+    }
+    // ordered behind everything queued on the context's stream (cube deltas with light)
+    CU(cudaMemcpyAsync(s->d_light_base, s->d_light, s->volume * 4, cudaMemcpyDeviceToDevice, s->ctx->stream));
+    CU(cudaStreamSynchronize(s->ctx->stream));
+    return AICB_OK;
+}
+
+aicb_status take_changes(aicb_scene *s, int32_t (*cubes)[3], uint8_t (*texels)[4], size_t cap, size_t *n_changed) {
+    if (!s->d_light_base) return aicb_fail(AICB_ERR_INVALID, "light change tracking is not enabled");
+    CU(cudaSetDevice(s->ctx->device));
+    aicb_ctx *c = s->ctx;
+    const uint32_t n_tiles = (uint32_t)((s->volume + LIGHT_TILE - 1) / LIGHT_TILE);
+    const int blocks = c->num_sms * 8;
+    k_diff_count<<<blocks, 256, 0, c->stream>>>(s->d_light, s->d_light_base, (uint32_t)s->volume, n_tiles, s->d_tile_count);
+    k_tile_scan<<<1, 1024, 0, c->stream>>>(s->d_tile_count, s->d_tile_off, n_tiles, s->d_scalars + SLOT_DIFFS);
+    uint32_t total = 0;
+    CU(cudaMemcpyAsync(&total, s->d_scalars + SLOT_DIFFS, 4, cudaMemcpyDeviceToHost, c->stream));
+    CU(cudaStreamSynchronize(c->stream));
+    CU(cudaGetLastError());
+    *n_changed = total;
+    if (total == 0 || total > cap) return AICB_OK;
+    if (s->changes_cap < total) {
+        if (s->d_changes) {
+            cudaFree(s->d_changes);
+            s->device_bytes -= s->changes_cap * 16;
+        }
+        s->d_changes = nullptr;
+        s->changes_cap = 0;
+        const size_t want = total < 4096 ? 4096 : (size_t)total + total / 2;
+        CU(cudaMalloc(&s->d_changes, want * 16));
+        s->changes_cap = want;
+        s->device_bytes += want * 16;
+    }
+    int32_t *d_cubes = (int32_t *)s->d_changes;
+    uint32_t *d_texels = s->d_changes + 3 * s->changes_cap;
+    k_diff_take<<<blocks, 256, 0, c->stream>>>(s->ds, s->d_light_base, n_tiles, s->d_tile_count, s->d_tile_off, d_cubes, d_texels);
+    CU(cudaMemcpyAsync(cubes, d_cubes, (size_t)total * 12, cudaMemcpyDeviceToHost, c->stream));
+    CU(cudaMemcpyAsync(texels, d_texels, (size_t)total * 4, cudaMemcpyDeviceToHost, c->stream));
+    CU(cudaStreamSynchronize(c->stream));
+    CU(cudaGetLastError());
+    return AICB_OK;
 }
 
 }  // namespace
@@ -1288,6 +1700,45 @@ aicb_status aicb_group_light_edit_and_propagate(aicb_group_scene *gs, const int3
     if (!gs || (n_edits && (!cubes || !new_ids))) return aicb_fail(AICB_ERR_INVALID, "NULL argument");
     return edit_and_relax(gs->scene, gs->group, cubes, new_ids, n_edits, epsilon, gs->light_stats, updates_done, max_diff,
                           nullptr);
+}
+
+aicb_status aicb_light_step(aicb_scene *s, const int32_t (*cubes)[3], const uint16_t *new_ids, size_t n_edits,
+                            uint8_t epsilon, uint64_t max_updates, double budget_us, aicb_light_updates *out) {
+    if (!s || (n_edits && (!cubes || !new_ids))) return aicb_fail(AICB_ERR_INVALID, "NULL argument");
+    return edit_and_relax({s}, nullptr, cubes, new_ids, n_edits, epsilon, nullptr, nullptr, nullptr, nullptr, &max_updates,
+                          budget_us, out);
+}
+
+aicb_status aicb_group_light_step(aicb_group_scene *gs, const int32_t (*cubes)[3], const uint16_t *new_ids,
+                                  size_t n_edits, uint8_t epsilon, uint64_t max_updates, double budget_us,
+                                  aicb_light_updates *out) {
+    if (!gs || (n_edits && (!cubes || !new_ids))) return aicb_fail(AICB_ERR_INVALID, "NULL argument");
+    return edit_and_relax(gs->scene, gs->group, cubes, new_ids, n_edits, epsilon, gs->light_stats, nullptr, nullptr,
+                          nullptr, &max_updates, budget_us, out);
+}
+
+aicb_status aicb_light_track_changes(aicb_scene *s, int enable) {
+    if (!s) return aicb_fail(AICB_ERR_INVALID, "NULL argument");
+    std::lock_guard<std::mutex> lock(s->ctx->mu);
+    return track_changes(s, enable);
+}
+
+aicb_status aicb_light_take_changes(aicb_scene *s, int32_t (*cubes)[3], uint8_t (*texels)[4], size_t cap,
+                                    size_t *n_changed) {
+    if (!s || !n_changed || (cap && (!cubes || !texels))) return aicb_fail(AICB_ERR_INVALID, "NULL argument");
+    std::lock_guard<std::mutex> lock(s->ctx->mu);
+    return take_changes(s, cubes, texels, cap, n_changed);
+}
+
+aicb_status aicb_group_light_track_changes(aicb_group_scene *gs, int enable) {
+    if (!gs) return aicb_fail(AICB_ERR_INVALID, "NULL argument");
+    return aicb_light_track_changes(gs->scene[0], enable);
+}
+
+aicb_status aicb_group_light_take_changes(aicb_group_scene *gs, int32_t (*cubes)[3], uint8_t (*texels)[4], size_t cap,
+                                          size_t *n_changed) {
+    if (!gs) return aicb_fail(AICB_ERR_INVALID, "NULL argument");
+    return aicb_light_take_changes(gs->scene[0], cubes, texels, cap, n_changed);
 }
 
 aicb_status aicb_group_light_download(aicb_group_scene *gs, int member, uint8_t (*out)[4], size_t n_texels) {

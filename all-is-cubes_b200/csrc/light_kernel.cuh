@@ -82,7 +82,8 @@ constexpr uint32_t LIGHT_TILE = 1024;   // cubes per queue tile (256 words of pe
 // The slots of LightParams::scalars, one propagation's counters in device memory.  A round's kernels read the round's
 // list length and priority from there, so rounds are queued back to back without a host round trip; a round whose
 // priority is already <= epsilon does nothing.  The per-round slots are reset before each round: [LIST_LEN, PRIORITY]
-// and [CHANGED, OVERFLOW]; the others accumulate over the propagation.
+// and [CHANGED, OVERFLOW]; the others accumulate over the propagation.  [TAKEN, QUEUE_MAX] are used only by the
+// capped rounds and the queue report of a step (aicb_light_step), SLOT_DIFFS only by aicb_light_take_changes.
 enum LightScalar : uint32_t {
     SLOT_LIST_LEN = 0,    // cubes gathered this round
     SLOT_PRIORITY = 1,    // highest queued priority this round
@@ -93,6 +94,11 @@ enum LightScalar : uint32_t {
     SLOT_WALK_NEXT = 7,   // the next list entry the compute walk hands out this round
     SLOT_MARK_NEXT = 8,   // the next `changed` entry the mark walk hands out this round
     SLOT_OVERFLOW = 9,    // entries of the overflow list this round
+    SLOT_TAKEN = 10,      // cubes the capped rounds of the step took so far, summed over the members (same in every member)
+    SLOT_BAND = 11,       // cubes of the round's band in the member's own tiles (a capped round; peers read it)
+    SLOT_QUEUED = 12,     // the step's queue report: queued cubes in the member's own tiles ...
+    SLOT_QUEUE_MAX = 13,  // ... and their highest priority
+    SLOT_DIFFS = 14,      // texels that differ from the change-tracking baseline
     LIGHT_SCALARS = 16    // slots allocated
 };
 

@@ -137,6 +137,20 @@ pub struct aicb_hit {
     pub face: i32,
 }
 
+/// `LightUpdatesInfo` (updater.rs:970-984) of one `aicb_light_step`, plus counters
+#[repr(C)]
+#[derive(Clone, Copy, Debug, Default)]
+pub struct aicb_light_updates {
+    pub update_count: u64,
+    pub queue_count: u64,
+    pub chart_node_visits: u64,
+    pub rounds: u32,
+    pub max_update_difference: u8,
+    pub max_queue_priority: u8,
+    pub _pad: [u8; 2],
+    pub device_ms: f32,
+}
+
 #[repr(C)]
 pub struct aicb_ctx {
     _opaque: [u8; 0],
@@ -232,6 +246,18 @@ unsafe extern "C" {
     pub fn aicb_group_light_download(gs: *mut aicb_group_scene, member: c_int, out: *mut [u8; 4], n_texels: usize) -> aicb_status;
     /// `member` -1: the group's totals; else that member's own counters.
     pub fn aicb_group_light_stats(gs: *const aicb_group_scene, member: c_int, out: *mut [u64; 4]) -> aicb_status;
+    /// `max_updates` u64::MAX / `budget_us` < 0: no limit; `out` may be null.
+    pub fn aicb_light_step(s: *mut aicb_scene, cubes: *const [i32; 3], new_ids: *const u16, n_edits: usize, epsilon: u8,
+                           max_updates: u64, budget_us: f64, out: *mut aicb_light_updates) -> aicb_status;
+    pub fn aicb_group_light_step(gs: *mut aicb_group_scene, cubes: *const [i32; 3], new_ids: *const u16, n_edits: usize,
+                                 epsilon: u8, max_updates: u64, budget_us: f64, out: *mut aicb_light_updates) -> aicb_status;
+    pub fn aicb_light_track_changes(s: *mut aicb_scene, enable: c_int) -> aicb_status;
+    /// Writes and consumes nothing when `*n_changed` (always the count) exceeds `cap`.
+    pub fn aicb_light_take_changes(s: *mut aicb_scene, cubes: *mut [i32; 3], texels: *mut [u8; 4], cap: usize,
+                                   n_changed: *mut usize) -> aicb_status;
+    pub fn aicb_group_light_track_changes(gs: *mut aicb_group_scene, enable: c_int) -> aicb_status;
+    pub fn aicb_group_light_take_changes(gs: *mut aicb_group_scene, cubes: *mut [i32; 3], texels: *mut [u8; 4], cap: usize,
+                                         n_changed: *mut usize) -> aicb_status;
 
     pub fn aicb_trace_rays(s: *mut aicb_scene, origin_dir: *const [f64; 6], n: usize, opt: *const aicb_options,
                            out_colorbuf: *mut [f32; 4], depth: *mut f64, hit: *mut aicb_hit, steps: *mut u32,

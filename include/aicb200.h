@@ -404,6 +404,52 @@ aicb_status aicb_light_download(aicb_scene *, uint8_t (*out)[4], size_t n_texels
  * term slots than the chain walk holds and took the overflow walk instead, out[3] 0. */
 aicb_status aicb_light_stats(const aicb_scene *, uint64_t out[4]);
 
+/* ---------------------------------------------------------------------------------------------
+ * Light propagation in budgeted steps, for a host that drives light once per tick (update_light_system,
+ * space/step.rs:340-368): each step relaxes until nothing above epsilon is queued or its budget is used up, and
+ * reports what is left in the queue.  The cubes whose light changed (SpaceChange::CubeLight) are listed on request.
+ * ------------------------------------------------------------------------------------------- */
+/* LightUpdatesInfo (space/light/updater.rs:970-984) of one step, plus counters.  40 bytes. */
+typedef struct aicb_light_updates {
+    uint64_t update_count;          /* compute_light calls applied by this step */
+    uint64_t queue_count;           /* cubes queued on return (queue byte > 0, any priority) */
+    uint64_t chart_node_visits;
+    uint32_t rounds;                /* relaxation rounds queued by this step (as aicb_light_stats out[2]) */
+    uint8_t  max_update_difference;
+    uint8_t  max_queue_priority;    /* highest queued Priority on return, 0 = empty (queue.rs:28-50 values) */
+    uint8_t  _pad[2];
+    float    device_ms;             /* CUDA-event time of the step (group: the slowest member's) */
+} aicb_light_updates;
+
+/* Mutation::set x n_edits (exactly as aicb_light_edit_and_propagate), then update_light_from_queue(budget)
+ * (updater.rs:181-291) down to epsilon, stopping when max_updates cube updates are done or the time budget is
+ * used up.  max_updates: UINT64_MAX = no limit, 0 = no relaxation (edits and the report only).
+ * budget_us < 0 = no time limit, 0 = no relaxation; a positive budget becomes an update cap (at least 1) through the
+ * scene's running estimate of device microseconds per cube update, which every step that updated a cube refines.
+ * With neither limit the step relaxes exactly as aicb_light_edit_and_propagate does.  A step stops between rounds:
+ * the cubes a round takes are the first ones of its priority band in index order.  out may be NULL; after a step
+ * aicb_light_stats reports its counters.  LightPhysics::None, NULL arrays with n_edits > 0, an invalid edit or a NaN
+ * budget is AICB_ERR_INVALID, and then nothing changed. */
+aicb_status aicb_light_step(aicb_scene *, const int32_t (*cubes)[3], const uint16_t *new_ids, size_t n_edits,
+                            uint8_t epsilon, uint64_t max_updates, double budget_us, aicb_light_updates *out);
+aicb_status aicb_group_light_step(aicb_group_scene *, const int32_t (*cubes)[3], const uint16_t *new_ids,
+                                  size_t n_edits, uint8_t epsilon, uint64_t max_updates, double budget_us,
+                                  aicb_light_updates *out);
+
+/* SpaceChange::CubeLight for a host that mirrors the light.  Enabling records the current light as the baseline
+ * (4 bytes per cube of device memory, freed when disabled).  take_changes lists every cube whose texel differs
+ * from the baseline, in increasing linear (Z-major) index, as world coordinates plus the current texel.  If the
+ * count is <= cap, it writes the list and moves the baseline of those cubes to the current value.  Otherwise it
+ * writes and consumes nothing.  *n_changed is always the count.  cubes / texels may be NULL only with cap == 0.
+ * Taking changes without tracking enabled is AICB_ERR_INVALID.  A group tracks member 0's replica; all replicas
+ * are identical on return from every light call. */
+aicb_status aicb_light_track_changes(aicb_scene *, int enable);
+aicb_status aicb_light_take_changes(aicb_scene *, int32_t (*cubes)[3], uint8_t (*texels)[4], size_t cap,
+                                    size_t *n_changed);
+aicb_status aicb_group_light_track_changes(aicb_group_scene *, int enable);
+aicb_status aicb_group_light_take_changes(aicb_group_scene *, int32_t (*cubes)[3], uint8_t (*texels)[4],
+                                          size_t cap, size_t *n_changed);
+
 #ifdef __cplusplus
 }
 #endif
